@@ -2,6 +2,7 @@
 """bench.py — AttU_Net 256x256 training throughput (images/s) on N B200s, one JSON line on rank 0.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--batch B] [--model NAME]
+                    [--dump-outputs DIR]
 
 A step = zero_grad -> forward -> BCEWithLogits -> backward -> (gradient all-reduce) -> clip_grad_norm_(1.0) ->
 AdamW step, i.e. the body of the reference's train() hot loop (utils/helpers.py:317-337) on synthetic
@@ -16,6 +17,12 @@ roofline : tcgen05 implicit-GEMM convolution kernel (fprop + dgrad launches): al
          the measured sustained bf16 peak in MEASURED_PEAKS.json.
 cpu_baseline / --impl reference : the oracle port of the reference (oracle/unet_oracle.py, pinned to the real
          reference by tests/golden) timed on the host cores, batch 4 per step (BASELINE.json configs[0]).
+reductions : every run of the B200 arm uses the library's deterministic-reduction mode (fixed-order sums instead of
+         atomics), so that the same arguments compute the same bits.  With atomics the summation order varies, and
+         AdamW turns the rounding noise of near-zero gradients (the conv biases ahead of BatchNorm) into steps of about
+         lr that spread to every weight: two runs would train different models.
+--dump-outputs DIR : after the timed steps, DIR/<name>.npy holds what the last of them computed (see output_arrays);
+         the inputs depend on the arguments alone, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -59,7 +66,36 @@ def parse():
                     help="1: weight-gradient kernels on a side stream, overlapping the memory-bound backward kernels")
     ap.add_argument("--graph", type=int, default=1,
                     help="capture the whole training step in a CUDA graph (single-GPU runs); 0 = eager launches")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss and the model state of the last timed step as DIR/<name>.npy (rank 0)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 path computed; it does not apply to --impl reference")
+    return args
+
+
+DUMP_BYTES = 64 << 20        # cap on what --dump-outputs writes
+DUMP_SAMPLE = 16384          # elements kept of a larger tensor
+
+
+def output_arrays(loss, model):
+    """What a caller of the training step receives: the step's loss and the state the step leaves in the model (parameters
+    and BatchNorm running statistics), as {name: float32 or float64 array}.  A tensor of more than DUMP_SAMPLE elements
+    is cut to a fixed, seeded sample of its flattened values, the same positions on every run."""
+    import numpy as np
+    import torch
+    out = {"loss": loss.detach().float().cpu().numpy()}
+    for k, v in model.state_dict().items():
+        v = v.detach()
+        if v.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(v.numel(), DUMP_SAMPLE, replace=False))
+            v = v.reshape(-1)[torch.from_numpy(idx).to(v.device)]
+        wide = v.dtype == torch.float64 or not v.is_floating_point()       # num_batches_tracked counts, fp64 state
+        out[k] = v.to(torch.float64 if wide else torch.float32).cpu().numpy()
+    assert sum(a.nbytes for a in out.values()) <= DUMP_BYTES
+    return out
 
 
 TRAFFIC_FILE = "r02f_traffic.json"      # ncu DRAM counters of one step of the default workload (tools/profile_step.py)
@@ -235,6 +271,7 @@ def run_b200(args):
     from b200seg.models import segmentation_models as M
     from b200seg.ddp import GradReducer
     from b200seg.utils.synthetic import xray_batch
+    from torchvision.models import WeightsEnum
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -252,8 +289,14 @@ def run_b200(args):
         dist.init_process_group("nccl", device_id=dev)
     _lib.check(_lib.load().b2_arch_check(), "b2_arch_check")
     K.set_wgrad_overlap(bool(args.wgrad_overlap))
+    K.set_deterministic(True)             # the same arguments compute the same bits (see "reductions" above)
 
     kw = {"t": args.t} if (args.t is not None and args.model != "AttentionUNet") else {}
+    def no_download(self, *args, **kwargs):
+        raise RuntimeError(f"{self} is not fetched: the benchmark uses random init")
+    # ResNetUnet: every pretrained-weight request fails as it does offline, so the model takes its seeded random-init
+    # fallback, never a downloaded or cached checkpoint, and the inputs depend on the arguments alone
+    WeightsEnum.get_state_dict = no_download
     torch.manual_seed(0)
     model = getattr(M, args.model)(**kw).to(dev, memory_format=torch.channels_last)   # helpers.py:243
     model.train()
@@ -297,13 +340,13 @@ def run_b200(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(k):
-            fn()
+            out = fn()
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms)
+        return float(ms), out
 
     # The package's own fast step (b200seg.engine.GraphedTrainStep — the same object utils.helpers.train() drives):
     # the first calls run eagerly (warm-up), then the whole step — forward, loss, backward, bucketed NCCL all-reduces,
@@ -343,12 +386,18 @@ def run_b200(args):
 
     l0 = _lib.launch_count
     sampler.mark_begin()
-    ms = timed(run_step, args.steps)
+    ms, loss = timed(run_step, args.steps)
     sampler.mark_end()
     launches = (_lib.launch_count - l0) if not graphed else launches_per_step * args.steps
     time.sleep(0.06)                      # let the sampler deliver the last row of the region
     clocks = sampler.stop() if rank == 0 else None
     _tick("timed region done")
+    if args.dump_outputs and rank == 0:   # now: the passes below train the model further
+        import numpy as np
+        out_dir = Path(args.dump_outputs)
+        out_dir.mkdir(parents=True, exist_ok=True)
+        for name, a in output_arrays(loss, model).items():
+            np.save(out_dir / f"{name}.npy", a)
 
     # end-to-end through the package API: every step's batch starts in pinned HOST memory (as DataLoader(pin_memory=True)
     # delivers it), PinnedPrefetcher copies batch i+1 on its copy stream while step i computes, the stepper copies it
@@ -372,7 +421,7 @@ def run_b200(args):
         xb, tb = next(e2e_iter)
         return float(stepper(xb, tb))
     e2e_step()
-    ms_e2e = timed(e2e_step, args.steps)
+    ms_e2e, _ = timed(e2e_step, args.steps)
     h2d_per_step = pre.h2d_bytes // (args.steps + 1)
     _tick("e2e done")
     # data-parallel sanity inside the measured run: after all those steps every replica must hold the same parameters
@@ -439,7 +488,8 @@ def run_b200(args):
                    "per_gpu_batch": B, "global_batch": B * world, "parallelism": f"dp{world}",
                    "l2": "working set per step (>10 GB of activations) far exceeds the 126 MB L2",
                    "model_kwargs": kw, "cuda_graph": graph is not None, "optimizer": args.optimizer,
-                   "wgrad_side_stream": bool(args.wgrad_overlap)},
+                   "wgrad_side_stream": bool(args.wgrad_overlap),
+                   "deterministic_reductions": K.deterministic_enabled()},
         "e2e": {"value": e2e, "unit": "images/s", "h2d_bytes_per_step": int(h2d_per_step),
                 "d2h_bytes_per_step": 4, "ms_per_step": ms_e2e / args.steps},
         "gpu_launches": launches,

@@ -18,6 +18,15 @@ for p in (str(ROOT), str(PKG)):
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a B200 (run with -m gpu on the GPU box)")
+    # ResNetUnet asks torchvision for the ImageNet ResNet-50 checkpoint, a download: every such request fails at once, as
+    # it does offline, so the tests use the model's seeded random-init fallback on every machine and none of them reaches
+    # the network or depends on what the user's torch cache holds
+    from torchvision.models import WeightsEnum
+
+    def no_download(self, *args, **kwargs):
+        raise RuntimeError(f"{self} is not fetched: the tests use random init")
+
+    WeightsEnum.get_state_dict = no_download
 
 
 def pytest_collection_modifyitems(config, items):

@@ -89,9 +89,7 @@ def test_aug_params_size_matches_header():
     assert C.sizeof(C.c_float) == 4
 
 
-def test_bench_clock_sampler_keeps_the_rows_of_the_timed_region():
-    """bench.py's nvidia-smi sampler starts before the warm-up and stamps its rows; only those inside the timed region
-    count (median clock, throttle reasons), with the rows around it as the fallback for a region shorter than one period."""
+def _load_bench():
     import importlib.util
     import sys
     spec = importlib.util.spec_from_file_location("bench_mod", ROOT / "bench.py")
@@ -101,6 +99,13 @@ def test_bench_clock_sampler_keeps_the_rows_of_the_timed_region():
         spec.loader.exec_module(bench)
     finally:
         sys.argv = argv
+    return bench
+
+
+def test_bench_clock_sampler_keeps_the_rows_of_the_timed_region():
+    """bench.py's nvidia-smi sampler starts before the warm-up and stamps its rows; only those inside the timed region
+    count (median clock, throttle reasons), with the rows around it as the fallback for a region shorter than one period."""
+    bench = _load_bench()
 
     class _Proc:
         def terminate(self):
@@ -127,6 +132,42 @@ def test_bench_clock_sampler_keeps_the_rows_of_the_timed_region():
     out = s.stop()
     assert out["samples"] == 2 and "under load" in out["window"]
     assert bench.ClockSampler(0).stop()["sm_mhz"] is None          # nvidia-smi unavailable
+
+
+@pytest.mark.parametrize("name", ["AttentionUNet", "R2U_Net", "R2AttU_Net", "ResNetUnet"])
+def test_bench_output_arrays_are_a_fixed_sample_within_budget(name):
+    """bench.py --dump-outputs: the loss and every state_dict entry of the model, float32 / float64, large tensors cut
+    to the same seeded positions on every run, the whole at most 64 MB"""
+    import warnings
+    from b200seg.models import segmentation_models as M
+    bench = _load_bench()
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        torch.manual_seed(0)
+        m = getattr(M, name)()
+    sd = m.state_dict()
+    out = bench.output_arrays(torch.tensor(0.25), m)
+    assert list(out) == ["loss"] + list(sd) and float(out["loss"]) == 0.25
+    assert all(a.dtype in (np.float32, np.float64) for a in out.values())
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    big = [k for k, v in sd.items() if v.numel() > bench.DUMP_SAMPLE]
+    assert big
+    for k in big:
+        n = sd[k].numel()
+        idx = np.sort(np.random.default_rng(0).choice(n, bench.DUMP_SAMPLE, replace=False))
+        assert np.array_equal(out[k], sd[k].reshape(-1).numpy()[idx]), k
+    again = bench.output_arrays(torch.tensor(0.25), m)
+    assert all(np.array_equal(out[k], again[k]) for k in out)
+    small = next(k for k, v in sd.items() if v.is_floating_point() and v.numel() <= bench.DUMP_SAMPLE)
+    assert np.array_equal(out[small], sd[small].numpy())
+
+
+def test_bench_rejects_zero_steps():
+    import subprocess
+    import sys
+    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=300)
+    assert r.returncode == 2 and "--steps" in r.stderr
 
 
 def test_bench_reference_arm_contract():

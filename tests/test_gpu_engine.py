@@ -186,3 +186,36 @@ def test_deferred_running_updates_match_immediate_ones():
     assert any(int(v) == 3 for k, v in ref.items() if "num_batches" in k)        # the shared BatchNorms: t + 1 = 3
     bad = [k for k in ref if not torch.equal(ref[k], got[k])]
     assert not bad, bad[:5]
+
+
+def test_bench_dumps_the_state_the_timed_steps_left(tmp_path):
+    """bench.py --steps K --dump-outputs DIR: K steps are timed, and DIR holds the loss and every state_dict entry the
+    last of them left; each BatchNorm has counted 3 eager warm-up steps + the capture step + the K timed steps, and a
+    second run with the same arguments dumps the same bits"""
+    import json
+    import subprocess
+    import sys
+    from pathlib import Path
+
+    import numpy as np
+    root = Path(__file__).resolve().parent.parent
+
+    def run(out):
+        cmd = [sys.executable, str(root / "bench.py"), "--steps", "5", "--warmup", "1", "--batch", "2", "--side", "64",
+               "--no-cpu-baseline", "--dump-outputs", str(out)]
+        r = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-3000:]
+        lines = [ln for ln in r.stdout.splitlines() if ln.startswith("{")]
+        assert len(lines) == 1
+        d = json.loads(lines[0])
+        assert d["steps"] == 5 and d["config"]["cuda_graph"] and d["config"]["deterministic_reductions"]
+        return {p.stem: np.load(p) for p in out.glob("*.npy")}
+
+    arrays, again = run(tmp_path / "a"), run(tmp_path / "b")
+    gold = np.load(root / "tests" / "golden" / "AttentionUNet.npz")
+    assert set(arrays) == {"loss"} | {str(k) for k in gold["keys"]}
+    assert all(a.dtype in (np.float32, np.float64) and np.isfinite(a).all() for a in arrays.values())
+    assert 0.0 < float(arrays["loss"]) < 10.0
+    counts = [float(a) for k, a in arrays.items() if k.endswith("num_batches_tracked")]
+    assert counts and set(counts) == {3 + 1 + 5}
+    assert set(again) == set(arrays) and all(np.array_equal(arrays[k], again[k]) for k in arrays)
