@@ -50,6 +50,11 @@ int b2_num_sms(void);
  * of ONE compute stream at a time; NULL switches the mode off.  b2_get_deterministic() -> 0 | 1. */
 int b2_set_deterministic(void* workspace, int64_t bytes);
 int b2_get_deterministic(void);
+/* The finish of that mode on its own: for each segment k < nseg (1..4), dsts[k][i] += the sum over the rows
+ * r = 0, 1, ..., rows-1, in that order and in fp64, of partial[r * row_stride + offsets[k] + i], for i < counts[k];
+ * dsts[k] is double when dst_f64[k] != 0 and float otherwise.  One launch for all segments. */
+int b2_det_finish(const double* partial, int64_t rows, int32_t row_stride, int32_t nseg, const int32_t* offsets,
+                  const int32_t* counts, void* const* dsts, const int32_t* dst_f64, b2_stream_t stream);
 
 /* The B200SEG_* environment switches (DESIGN.md section 10) are read once and cached behind a mutex; call this after
  * changing the environment of a running process (tests do) to have them re-read. */

@@ -85,6 +85,7 @@ SIGNATURES = {
     "b2_arch_check": (C.c_int, []),
     "b2_num_sms": (C.c_int, []),
     "b2_set_deterministic": (C.c_int, [_vp, _i64]),
+    "b2_det_finish": (C.c_int, [_vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
     "b2_get_deterministic": (C.c_int, []),
     "b2_reload_env": (C.c_int, []),
     "b2_conv_fprop": (C.c_int, [C.POINTER(ConvArgs), _vp]),

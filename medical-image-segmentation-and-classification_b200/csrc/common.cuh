@@ -105,15 +105,29 @@ int encode_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_
 // Deterministic-reduction mode (b2_set_deterministic, include/b200seg.h).  Kernels whose last step is a cross-block
 // atomicAdd write ONE ROW of per-block partials into the registered workspace instead; det_finish adds the rows to the
 // destination in block order.  With the mode off (`partial == nullptr`) the kernels use their atomics.
+// The rows are not cleared: a producer writes every slot of its rows exactly once, or zeroes its own rows itself, and
+// only after its pdl_wait() — every reduction reuses the start of the workspace, and the previous finish may still
+// be reading it until then.
 // ---------------------------------------------------------------------------------------------
 struct DetBuf {
   double* partial;   // [rows][n] or nullptr
   int n;             // row length in doubles
 };
-// Reserve (and zero) rows*n doubles of the workspace for a launch on `stream`.  out->partial stays nullptr when the
-// mode is off.  Consecutive reservations of ONE entry point may coexist (`keep` = doubles already reserved by it).
+// Reserve rows*n doubles of the workspace for a launch on `stream`.  out->partial stays nullptr when the mode is
+// off.  Consecutive reservations of ONE entry point may coexist (`keep` = doubles already reserved by it).
 int det_begin(DetBuf* out, long long rows, int n, cudaStream_t stream, long long keep = 0);
-// dst[i] += sum over rows r (in order) of partial[r * row_stride + i], i < count
+// dst[i] += sum over rows r (in order) of partial[r * row_stride + offset + i], i < count, for up to kDetMaxSeg
+// segments of the same rows in ONE launch (dst double when f64, float otherwise)
+static constexpr int kDetMaxSeg = 4;
+struct DetSeg {
+  int offset;
+  int count;
+  void* dst;
+  int f64;
+};
+inline DetSeg det_seg(int offset, int count, double* dst) { return DetSeg{offset, count, dst, 1}; }
+inline DetSeg det_seg(int offset, int count, float* dst) { return DetSeg{offset, count, dst, 0}; }
+int det_finish(const double* partial, long long rows, int row_stride, const DetSeg* seg, int nseg, cudaStream_t stream);
 int det_finish(const double* partial, long long rows, int row_stride, int count, double* dst, cudaStream_t stream);
 int det_finish(const double* partial, long long rows, int row_stride, int count, float* dst, cudaStream_t stream);
 bool det_enabled();

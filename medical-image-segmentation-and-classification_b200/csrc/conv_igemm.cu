@@ -451,6 +451,13 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
     float* s_bias = s_bias0 + g * 256;
     float* s_psi = s_psi0 + g * 256;
     const int bar_id = 1 + g;
+    if (p.stats_partial != nullptr) {
+      // the flushes below add into this group's row, and a CTA may never meet some n-tile: zero the row first (after
+      // pdl_enter above — the previous finish may read the workspace until then), then sync the group
+      double* srow = p.stats_partial + (size_t)(blockIdx.x * G + g) * (2 * p.cout);
+      for (int i = et; i < 2 * p.cout; i += 128) srow[i] = 0.0;
+      asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");
+    }
     const int quad = warp & 3;                 // TMEM lane quadrant this warp may access
     const int row = quad * 32 + lane;          // accumulator row == pixel within the tile
     const int wl = row % p.Wb;

@@ -388,9 +388,8 @@ extern "C" int b2_head_bwd(const float* dy, const void* x, int32_t ldx, int64_t 
 #undef B2_HEAD_BWD
   B2_LAUNCH_CHECK();
   if (det.partial) {
-    rc = det_finish(det.partial, grid, det.n, cout * cin, dw, (cudaStream_t)stream);
-    if (rc) return rc;
-    return det_finish(det.partial + cout * cin, grid, det.n, cout, db, (cudaStream_t)stream);
+    const DetSeg seg[2] = {det_seg(0, cout * cin, dw), det_seg(cout * cin, cout, db)};
+    return det_finish(det.partial, grid, det.n, seg, 2, (cudaStream_t)stream);
   }
   return B2_OK;
 }

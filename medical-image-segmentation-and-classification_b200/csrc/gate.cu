@@ -616,11 +616,8 @@ extern "C" int b2_gate_psi_bwd_reduce(const float* dsig, const void* q, const vo
   }
   B2_LAUNCH_CHECK();
   if (det.partial) {
-    rc = det_finish(det.partial, grid, det.n, 4 * fint, sums, (cudaStream_t)stream);
-    if (rc) return rc;
-    rc = det_finish(det.partial + 4 * fint, grid, det.n, fint, dwpsi, (cudaStream_t)stream);
-    if (rc) return rc;
-    return det_finish(det.partial + 5 * fint, grid, det.n, 1, dbpsi, (cudaStream_t)stream);
+    const DetSeg seg[3] = {det_seg(0, 4 * fint, sums), det_seg(4 * fint, fint, dwpsi), det_seg(5 * fint, 1, dbpsi)};
+    return det_finish(det.partial, grid, det.n, seg, 3, (cudaStream_t)stream);
   }
   return B2_OK;
 }

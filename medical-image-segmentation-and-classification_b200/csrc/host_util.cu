@@ -74,6 +74,7 @@ bool det_enabled() {
 }
 
 int det_begin(DetBuf* out, long long rows, int n, cudaStream_t stream, long long keep) {
+  (void)stream;
   out->partial = nullptr;
   out->n = n;
   double* ws;
@@ -84,31 +85,117 @@ int det_begin(DetBuf* out, long long rows, int n, cudaStream_t stream, long long
              "deterministic workspace too small: need %lld B, have %lld B (b2_set_deterministic)",
              (keep + need) * 8, cap * 8);
   out->partial = ws + keep;
-  B2_CHECK_CUDA(cudaMemsetAsync(out->partial, 0, (size_t)need * sizeof(double), stream));
   return B2_OK;
 }
 
-template <typename T>
-__global__ void det_finish_kernel(const double* __restrict__ partial, long long rows, int row_stride, int count,
-                                  T* __restrict__ dst) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= count) return;
-  double s = 0.0;
-  for (long long r = 0; r < rows; ++r) s += partial[r * row_stride + i];     // fixed order: bit-reproducible
-  dst[i] = (T)((double)dst[i] + s);
+// Finish: one block per slab of up to 32 consecutive columns of one segment.  The block streams chunks of the slab's
+// rows (kFinChunk doubles: 96 rows of 32 columns, 3072 rows of one column) through two shared-memory buffers, every
+// thread holding kFinChunk / kFinThreads independent loads in flight, while one lane per column adds the previous
+// chunk in row order.  The sum of a column is the same chain of fp64 additions as a serial loop over the rows, so the
+// result does not depend on the slab width or the chunking; the loads no longer sit on that chain.
+static constexpr int kFinThreads = 256;
+static constexpr int kFinChunk = 3072;
+static constexpr int kFinLoads = kFinChunk / kFinThreads;
+
+struct DetFinishJob {
+  const double* partial;
+  long long rows;
+  int row_stride;
+  int nseg;
+  DetSeg seg[kDetMaxSeg];
+  int first_block[kDetMaxSeg + 1];    // blocks [first_block[s], first_block[s + 1]) finish segment s
+};
+
+__global__ void __launch_bounds__(kFinThreads) det_finish_kernel(DetFinishJob j) {
+  __shared__ double buf[2][kFinChunk];
+  pdl_enter();          // the producer has completed: its partial rows are complete and visible
+  int s = 0;
+  while (s + 1 < j.nseg && (int)blockIdx.x >= j.first_block[s + 1]) ++s;
+  const DetSeg sg = j.seg[s];
+  const int c0 = ((int)blockIdx.x - j.first_block[s]) * 32;
+  const int w = sg.count - c0 < 32 ? sg.count - c0 : 32;        // columns of this slab
+  const int ch = kFinChunk / w;                                  // rows per chunk
+  const int per = ch * w;
+  const long long rows = j.rows;
+  const double* src = j.partial + sg.offset + c0;
+  // element e = k * kFinThreads + threadIdx.x of a chunk is (row e / w, column e % w): a warp reads whole rows
+  int er[kFinLoads], eo[kFinLoads];
+#pragma unroll
+  for (int k = 0; k < kFinLoads; ++k) {
+    const int e = k * kFinThreads + (int)threadIdx.x;
+    er[k] = e < per ? e / w : INT32_MAX;
+    eo[k] = e < per ? er[k] * j.row_stride + (e - er[k] * w) : 0;
+  }
+  double v[kFinLoads];
+  auto load = [&](long long r0) {
+    const double* base = src + r0 * j.row_stride;
+#pragma unroll
+    for (int k = 0; k < kFinLoads; ++k) v[k] = r0 + er[k] < rows ? __ldg(base + eo[k]) : 0.0;
+  };
+  auto stash = [&](double* b) {
+#pragma unroll
+    for (int k = 0; k < kFinLoads; ++k)
+      if (k * kFinThreads + (int)threadIdx.x < per) b[k * kFinThreads + threadIdx.x] = v[k];
+  };
+  const long long nchunks = (rows + ch - 1) / ch;
+  load(0);
+  stash(buf[0]);
+  __syncthreads();
+  double acc = 0.0;
+  for (long long q = 0; q < nchunks; ++q) {
+    if (q + 1 < nchunks) load((q + 1) * ch);                     // in flight while the chunk q is added
+    if ((int)threadIdx.x < w) {
+      const double* b = buf[q & 1] + threadIdx.x;
+      const int n = rows - q * ch < ch ? (int)(rows - q * ch) : ch;
+#pragma unroll 8
+      for (int r = 0; r < n; ++r) acc += b[r * w];
+    }
+    if (q + 1 < nchunks) stash(buf[(q + 1) & 1]);                // buffer (q + 1) & 1 was last read before the
+    __syncthreads();                                             // previous barrier
+  }
+  if ((int)threadIdx.x < w) {
+    const int i = c0 + (int)threadIdx.x;
+    if (sg.f64) {
+      double* d = static_cast<double*>(sg.dst);
+      d[i] = d[i] + acc;
+    } else {
+      float* d = static_cast<float*>(sg.dst);
+      d[i] = (float)((double)d[i] + acc);
+    }
+  }
 }
 
+int det_finish(const double* partial, long long rows, int row_stride, const DetSeg* seg, int nseg,
+               cudaStream_t stream) {
+  B2_REQUIRE(nseg >= 1 && nseg <= kDetMaxSeg && rows >= 1, B2_ERR_SHAPE, "det_finish: %d segments, %lld rows",
+             nseg, rows);
+  DetFinishJob j;
+  j.partial = partial;
+  j.rows = rows;
+  j.row_stride = row_stride;
+  j.nseg = nseg;
+  int blocks = 0;
+  for (int s = 0; s < nseg; ++s) {
+    B2_REQUIRE(seg[s].count >= 0 && seg[s].offset >= 0 && seg[s].offset + seg[s].count <= row_stride, B2_ERR_SHAPE,
+               "det_finish: segment %d (offset %d, count %d) outside a row of %d", s, seg[s].offset, seg[s].count,
+               row_stride);
+    j.seg[s] = seg[s];
+    j.first_block[s] = blocks;
+    blocks += (seg[s].count + 31) / 32;
+  }
+  j.first_block[nseg] = blocks;
+  if (blocks == 0) return B2_OK;
+  B2_CHECK_CUDA(launch_chain(det_finish_kernel, dim3(blocks), dim3(kFinThreads), (size_t)0, stream, 1,
+                             rows * row_stride * (long long)sizeof(double), j));
+  return B2_OK;
+}
 int det_finish(const double* partial, long long rows, int row_stride, int count, double* dst, cudaStream_t stream) {
-  if (count <= 0) return B2_OK;
-  det_finish_kernel<double><<<(count + 127) / 128, 128, 0, stream>>>(partial, rows, row_stride, count, dst);
-  B2_LAUNCH_CHECK();
-  return B2_OK;
+  const DetSeg s = det_seg(0, count, dst);
+  return det_finish(partial, rows, row_stride, &s, 1, stream);
 }
 int det_finish(const double* partial, long long rows, int row_stride, int count, float* dst, cudaStream_t stream) {
-  if (count <= 0) return B2_OK;
-  det_finish_kernel<float><<<(count + 127) / 128, 128, 0, stream>>>(partial, rows, row_stride, count, dst);
-  B2_LAUNCH_CHECK();
-  return B2_OK;
+  const DetSeg s = det_seg(0, count, dst);
+  return det_finish(partial, rows, row_stride, &s, 1, stream);
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -184,6 +271,15 @@ int b2_set_deterministic(void* workspace, int64_t bytes) {
 }
 
 int b2_get_deterministic(void) { return b2::det_enabled() ? 1 : 0; }
+
+int b2_det_finish(const double* partial, int64_t rows, int32_t row_stride, int32_t nseg, const int32_t* offsets,
+                  const int32_t* counts, void* const* dsts, const int32_t* dst_f64, b2_stream_t stream) {
+  B2_REQUIRE(nseg >= 1 && nseg <= b2::kDetMaxSeg, B2_ERR_SHAPE, "b2_det_finish: %d segments (1..%d)", nseg,
+             b2::kDetMaxSeg);
+  b2::DetSeg seg[b2::kDetMaxSeg];
+  for (int s = 0; s < nseg; ++s) seg[s] = {offsets[s], counts[s], dsts[s], dst_f64[s] != 0 ? 1 : 0};
+  return b2::det_finish(partial, rows, row_stride, seg, nseg, (cudaStream_t)stream);
+}
 
 int b2_reload_env(void) {
   std::lock_guard<std::mutex> lk(b2::g_env_mu);
