@@ -164,17 +164,9 @@ class Recurrent_block(nn.Module):
                                           share_count=n_uses)
         if self.t == 0:
             raise ValueError("Recurrent_block needs t >= 1 (the reference leaves x1 undefined for t = 0)")
-        from .ops_infer import inference_mode
-        if ops._RECURRENT_PASS and torch.is_grad_enabled() and x.requires_grad and not inference_mode(self.conv[1]):
-            # training: x travels along the applications as a pass-through, so that its t + 1 gradients meet inside
-            # the first application's dgrad instead of in autograd's accumulation passes (ops._CbaPass)
-            s, xp = ops.conv_bn_act_pass(x, x, self.conv[0], self.conv[1], 0, n_uses, True)
-            for i in range(self.t - 1):
-                s, xp = ops.conv_bn_act_pass(s, xp, self.conv[0], self.conv[1], i + 1, n_uses, False)
-        else:
-            s = f(x, x, 0)                    # x + f(x)
-            for i in range(self.t - 1):
-                s = f(s, x, i + 1)            # x + f(x + x1)
+        s = f(x, x, 0)                        # x + f(x)
+        for i in range(self.t - 1):
+            s = f(s, x, i + 1)                # x + f(x + x1)
         x1 = f(s, None, self.t)
         return ops.to_nchw(x1) if ext else x1
 

@@ -320,9 +320,8 @@ _SHARED_DW = {}      # (weight address, device) -> fp32 gradient buffer of a sha
 @custom_op("b200seg::conv_bn_act_bwd", mutates_args=())
 def conv_bn_act_bwd(dy: Tensor, x0: Tensor, x1: Optional[Tensor], x4: Tensor, weight: Tensor, z: Tensor,
                     coef: Tensor, gamma: Tensor, relu: bool, training: bool, need_dx0: bool, need_dx1: bool,
-                    has_bias: bool, share_index: int = 0, share_count: int = 1,
-                    dx_add: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
-    """dx_add: a gradient x0 received on another path, added to dx0 in the dgrad epilogue (conv_bn_act_pass)"""
+                    has_bias: bool, share_index: int = 0,
+                    share_count: int = 1) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
     cout, cin, k, _ = weight.shape
     dev = dy.device
     res = K.bn_bwd(_c(dy), z, coef, gamma, relu=relu, training=training, want_dbias=has_bias)
@@ -340,8 +339,7 @@ def conv_bn_act_bwd(dy: Tensor, x0: Tensor, x1: Optional[Tensor], x4: Tensor, we
         if need_dx0 or need_dx1:
             _, wd = K.packed(weight, want_dgrad=True)
             if need_dx0:
-                dx0 = K.conv_igemm(dz, wd, c0, k, row_offset=0, dgrad=True,
-                                   addend=_c(dx_add) if dx_add is not None else None)
+                dx0 = K.conv_igemm(dz, wd, c0, k, row_offset=0, dgrad=True)
             if need_dx1 and x1 is not None:
                 dx1 = K.conv_igemm(dz, wd, x1.shape[3], k, row_offset=c0, dgrad=True)
         with K.wgrad_stream(dz, x0, x1, allow=K.grad_is_stolen(weight)):
@@ -394,60 +392,6 @@ def _cba_backward(ctx, dy, *_unused):
 conv_bn_act.register_autograd(_cba_backward, setup_context=_cba_setup)
 
 
-class _CbaPass(torch.autograd.Function):
-    """(x + act(bn(conv(v))), x) — one application of Recurrent_block's shared conv (R2U_Net.py:15-20) that hands the next
-    application its addend x as a pass-through output.  x is the addend of every application but the last and the conv
-    input of the first, so autograd used to sum t + 1 full-size gradients for it in separate ATen passes; here the
-    identity gradients travel back along the pass-through chain (one b2_add per link) and, in the first application
-    (`same`: v is x), join the conv-input gradient inside the dgrad epilogue."""
-
-    @staticmethod
-    def forward(ctx, v, x, weight, bias, gamma, beta, rm, rv, training, eps, relu, share_index, share_count, same):
-        y, z, coef, stats, x4 = conv_bn_act(v, None, weight, bias, gamma, beta, rm, rv, training, eps, relu, x,
-                                            share_index, share_count)
-        ctx.save_for_backward(_c(v), x4, weight, z, coef, gamma)
-        ctx.cfg = (relu, training, bias is not None, share_index, share_count, same)
-        ctx.set_materialize_grads(False)
-        ctx.mark_non_differentiable(stats)
-        return y, x, stats
-
-    @staticmethod
-    def backward(ctx, dy, dxp, _dstats):
-        v, x4, weight, z, coef, gamma = ctx.saved_tensors
-        relu, training, has_bias, share_index, share_count, same = ctx.cfg
-        none12 = (None,) * 8
-        if dy is None:                         # the application's own output was not used
-            return (None, dxp, None, None, None, None) + none12
-        ident = _c(dy) if dxp is None else K.add(_c(dy), _c(dxp))      # d(addend) = d(output), plus the chain so far
-        need_v = bool(ctx.needs_input_grad[0])
-        dx0, _dx1, dw, db, dgamma, dbeta = conv_bn_act_bwd(dy, v, None, x4, weight, z, coef, gamma, relu, training,
-                                                           need_v, False, has_bias, share_index, share_count,
-                                                           ident if (same and need_v) else None)
-        gv = dx0 if need_v else None
-        gx = None if same else ident
-        return (gv, gx, _dw_as_param_grad(dw, weight) if dw.numel() > 0 else None, db if has_bias else None, dgamma,
-                dbeta) + none12
-
-
-# Off by default: measured neutral on the R2 models (R2AttU_Net(t=2) b32 39.8 vs 40.0 ms, R2U_Net 37.7 vs 37.3 ms) — the
-# ATen accumulation passes it removes were already hidden behind the weight-gradient stream, while the addend it adds
-# to the first application's dgrad sits on the critical path.  B200SEG_RECURRENT_PASS=1 switches it on.
-_RECURRENT_PASS = os.environ.get("B200SEG_RECURRENT_PASS", "0") == "1"
-
-
-def conv_bn_act_pass(v: Tensor, x: Tensor, conv: torch.nn.Conv2d, bn: torch.nn.BatchNorm2d, share_index: int,
-                     share_count: int, same: bool) -> Tuple[Tensor, Tensor]:
-    """-> (x + relu(bn(conv(v))), x as the tensor the next application should take as its addend)"""
-    training = bn.training or bn.running_mean is None
-    y, xp, stats = _CbaPass.apply(v, x, conv.weight, conv.bias, bn.weight, bn.bias, bn.running_mean, bn.running_var,
-                                  training, float(bn.eps), True, share_index, share_count, same)
-    if training:
-        n, h, w, _ = y.shape
-        bn_update_running_(stats.detach(), n * h * w, float(bn.momentum), bn.running_mean, bn.running_var,
-                           bn.num_batches_tracked)
-    return y, xp
-
-
 @custom_op("b200seg::bn_update_running_", mutates_args=("running_mean", "running_var", "num_batches_tracked"))
 def bn_update_running_(stats: Tensor, count: int, momentum: float, running_mean: Tensor, running_var: Tensor,
                        num_batches_tracked: Tensor) -> None:
@@ -482,8 +426,6 @@ def conv_bn_act_module(x, conv: torch.nn.Conv2d, bn: torch.nn.BatchNorm2d, relu:
 # the only numerical difference is that the 3x3 taps are summed in fp32 before the bf16 rounding of the weights.
 # ----------------------------------------------------------------------------------------------------------
 _PHASES = ((0, 0), (0, 1), (1, 0), (1, 1))
-_UPFOLD_MERGED = os.environ.get("B200SEG_UPFOLD_MERGED", "1") != "0"     # 0: four launches per direction (A/B switch)
-_UPFOLD_WGRAD_MERGED = os.environ.get("B200SEG_UPFOLD_WGRAD_MERGED", "1") != "0"   # 0: four weight-gradient launches
 
 
 @custom_op("b200seg::upconv_bn_act", mutates_args=())
@@ -497,7 +439,7 @@ def upconv_bn_act(x: Tensor, weight: Tensor, bias: Optional[Tensor], gamma: Tens
     stats = K.zeros_scratch((2, cout), _F64, dev) if training else torch.empty((0,), dtype=_F64, device=dev)
     wf, _ = K.packed(weight, "upfold")
     z = K.new_act(n, 2 * h, 2 * w, cout, dev)
-    if _UPFOLD_MERGED and cout % 64 == 0 and cin % 64 == 0:
+    if cout % 64 == 0 and cin % 64 == 0:
         # all four phase convolutions in ONE launch (the phase is an extra tile dimension, pixel-shuffle TMA stores)
         K.conv_igemm(x, wf.view(16, cout, cin), cout, 2, bias=bias, stats=stats if training else None, out=z, fold=1,
                      alg_scale=2.25)
@@ -533,7 +475,7 @@ def upconv_bn_act_bwd(dy: Tensor, x: Tensor, weight: Tensor, z: Tensor, coef: Te
     if need_dx:
         _, wd = K.packed(weight, "upfold", want_dgrad=True)
         dx = K.new_act(n, h, w, cin, dev)
-        if _UPFOLD_MERGED and cout % 64 == 0 and cin % 64 == 0:
+        if cout % 64 == 0 and cin % 64 == 0:
             # the four phases as ONE K loop of 16 taps over the sub-lattices of dz: one launch, one epilogue per tile
             K.conv_igemm(dz, wd.view(16, cin, cout), cin, 2, out=dx, dgrad=True, fold=2, alg_scale=2.25)
         else:
@@ -547,7 +489,7 @@ def upconv_bn_act_bwd(dy: Tensor, x: Tensor, weight: Tensor, z: Tensor, coef: Te
     with K.wgrad_stream(dz, x, allow=K.grad_is_stolen(weight)):
         dweff = torch.empty((4, cout, 4, cin), dtype=torch.float32, device=dev)
         # all four phases in ONE launch (every X row fetched once per filter row, the two column phases share it)
-        merged = _UPFOLD_WGRAD_MERGED and (cout == 64 or cout % 128 == 0) and cin % 64 == 0 and \
+        merged = (cout == 64 or cout % 128 == 0) and cin % 64 == 0 and \
             K.conv_wgrad(dz, x, 2, out=dweff, dy_mul=2, fold=True, alg_scale=2.25) is not None
         if not merged:
             for ph, (a, b) in enumerate(_PHASES):

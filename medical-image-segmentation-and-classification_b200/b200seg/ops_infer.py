@@ -65,9 +65,8 @@ def upconv_bn_act_infer(x: Tensor, weight: Tensor, bias: Optional[Tensor], gamma
     n, h, w, _ = x.shape
     wf, bf = _folded(weight, bias, gamma, beta, running_mean, running_var, eps, True)
     y = K.new_act(n, 2 * h, 2 * w, cout, x.device)
-    from . import ops as _ops
     cin = x.shape[3]
-    if _ops._UPFOLD_MERGED and cout % 64 == 0 and cin % 64 == 0:
+    if cout % 64 == 0 and cin % 64 == 0:
         K.conv_igemm(x, wf.view(16, cout, cin), cout, 2, bias=bf, relu=relu, out=y, fold=1)
     else:
         for ph, (a, b) in enumerate(_PHASES):

@@ -211,7 +211,7 @@ __device__ __forceinline__ void tma_load_5d(void* smem, const CUtensorMap* tm, u
       "l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
       : "memory");
 }
-// ---- thread-block clusters: multicast TMA loads (same smem offset + same mbarrier offset in every CTA of the mask)
+// ---- thread-block clusters
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -219,33 +219,6 @@ __device__ __forceinline__ uint32_t cluster_ctarank() {
 }
 __device__ __forceinline__ void cluster_sync_all() {     // every thread of every CTA in the cluster
   asm volatile("barrier.cluster.arrive.aligned;\n\tbarrier.cluster.wait.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tma_load_3d_mc(void* smem, const CUtensorMap* tm, uint64_t* bar, int c0, int c1,
-                                               int c2, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster "
-      "[%0], [%1, {%4, %5, %6}], [%2], %3;"
-      ::"r"(smem_u32(smem)), "l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(bar)), "h"(mask), "r"(c0), "r"(c1),
-      "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_4d_mc(void* smem, const CUtensorMap* tm, uint64_t* bar, int c0, int c1,
-                                               int c2, int c3, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster "
-      "[%0], [%1, {%4, %5, %6, %7}], [%2], %3;"
-      ::"r"(smem_u32(smem)), "l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(bar)), "h"(mask), "r"(c0), "r"(c1),
-      "r"(c2), "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_5d_mc(void* smem, const CUtensorMap* tm, uint64_t* bar, int c0, int c1,
-                                               int c2, int c3, int c4, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster "
-      "[%0], [%1, {%4, %5, %6, %7, %8}], [%2], %3;"
-      ::"r"(smem_u32(smem)), "l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(bar)), "h"(mask), "r"(c0), "r"(c1),
-      "r"(c2), "r"(c3), "r"(c4)
-      : "memory");
 }
 // ---- CTA pairs (tcgen05 cta_group::2): the two CTAs of a 2-cluster feed ONE M = 256 MMA issued by the rank-0 CTA.
 // Both CTAs load their own operand slices into their own shared memory, but the completion bytes are signalled on the
@@ -347,12 +320,6 @@ __device__ __forceinline__ void umma_commit_pair(uint64_t* bar, uint16_t mask) {
 // Arrive on an mbarrier when all previously issued tcgen05.mma of this thread have completed.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-// Same, arriving on the mbarrier at this smem offset in every CTA of `mask` (smem slots shared by multicast loads).
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"(mask)
                : "memory");
 }
 // 32 lanes x 32 consecutive fp32 columns: thread i of the warp gets TMEM lane (base_lane + i).

@@ -22,8 +22,11 @@
 // Double-M work items (BLOCK_N <= 128, large layers): two consecutive m-tiles share every weight stage — two A slots
 // per stage, four accumulators in TMEM, one epilogue group per tile.  The kernel is bound by the bytes each SM pulls
 // through the L2 -> SM fabric, and the weight tile is 75 % of them at N <= 128; sharing it is worth 14-29 % per layer.
-// Optional clusters (B200SEG_CLUSTER=2|4, off by default: no measured gain): the CTAs of a cluster work on
-// consecutive m-tiles of one n-tile and share every weight tile, each fetching 1/cluster of its rows and multicasting.
+// Clusters of 2 or 4 CTAs that multicast the weight tiles to each other were built and removed: no change at 2 CTAs,
+// slower at 4 (the multicast does not relieve what bounds these tiles).
+// A Cout = 64 "row-pair" mode (two output rows per tile, stacked taps, N = 128 MMAs) was built and removed: isolated
+// 64->64 @256^2 0.390 -> 0.366 ms, but inside the training step, where the weight gradients load the same L2 -> SM
+// fabric, the gain vanished.
 // CTA pairs (cta_group::2, IgemmParams::pair): the two CTAs of a 2-cluster share one M = 256 MMA, each holding its own
 // 128-pixel activation tile and half of the weight rows, which halves the weight bytes every SM pulls through the
 // L2 -> SM fabric without needing a second set of accumulators (the N = 256 layers fill TMEM with two buffers already).
@@ -50,24 +53,16 @@ struct IgemmParams {
   int taps;           // 1 or 9
   int cb0, cb1;       // 64-channel blocks in source 0 / 1
   int block_n, stages, num_k_iters;
-  int cout, n_tiles, m_tiles, m_stride;
-  int halo, base_off_mode;
+  int cout, n_tiles, m_tiles;
+  int halo;
   int dm;             // "double-M" mode: a work item is TWO consecutive m-tiles that share every weight stage (two A
                       // slots per stage, four accumulators in TMEM): halves the weight bytes a CTA pulls through the
                       // L2 -> SM fabric per FLOP.  BLOCK_N <= 128.
-  int rp;             // row-pair mode (Cout == 64, halo geometry): a tile is 128 pixels of TWO output rows; accumulator
-                      // columns 0..63 = row h0+1, 64..127 = row h0; every input row h0-1+j (j = 0..3) meets the stacked
-                      // taps [W(j-1, s) ; W(j, s)] (one strided TMA box, out-of-range filter rows zero-filled), so the
-                      // MMAs are N = 128 instead of N = 64 and 4 instead of 6 activation rows are fetched per two tiles
   int stride, ksize, pad_h, pad_w;
-  long long y_sn, y_sh, y_sw;   // element strides of the output pixel grid (strided placement for ConvT)
   int a_stage_bytes, b_stage_bytes, a_tx_bytes;
-  int tma_store;
   int epi_groups;     // 1 or 2 epilogue warp groups (two staging tiles)
   int ctile_bytes;    // bytes of one staging tile (128 x block_n bf16; at least one 64-channel panel in gate mode)
   int debug_skip;     // timing experiments only (B200SEG_DEBUG_SKIP): 1 = no TMA loads, 2 = no MMAs, 4 = no drain
-  int cluster;        // CTAs per cluster (1, 2 or 4): they work on consecutive m-tiles of one n-tile and share the
-                      // weight tiles, each CTA fetching 1/cluster of the rows and multicasting them
   int fold;           // folded-UpConv launches (AttentionUNet.py:15-27 as four 2x2 phase convolutions) merged into ONE:
                       //   1 = fprop: the phase (a, b) is an extra tile dimension; tile t belongs to phase t / m_tiles_phase,
                       //       uses weight taps 4*phase .. 4*phase+3 with tap offsets (u - (1-a), v - (1-b)) and stores to
@@ -88,12 +83,10 @@ struct IgemmParams {
                       // carries activations.  The Cout = 64 layers at 256^2 were bound by the L2 -> SM fabric
                       // (64->64: 51 KB of activations + 36 KB of weights per 128-pixel tile at ~10 TB/s chip-wide).
   int wres_bytes;     // bytes of the resident slab (this CTA's half in pair mode)
-  int pair;           // CTA-pair mode (cluster == 2): ONE tcgen05.mma.cta_group::2 with M = 256 covers the two m-tiles of
-                      // the pair; each CTA stages its own activation tile and HALF of the weight rows in its own shared
-                      // memory (no multicast: each SM receives half the weight bytes), the rank-0 CTA issues the MMAs,
-                      // every CTA drains its own 128 accumulator rows
-  __nv_bfloat16* y;
-  int ldy;
+  int pair;           // CTA-pair mode (2-CTA clusters, kernel instantiation kPair): ONE tcgen05.mma.cta_group::2 with
+                      // M = 256 covers the two m-tiles of the pair; each CTA stages its own activation tile and HALF of
+                      // the weight rows in its own shared memory (each SM receives half the weight bytes), the rank-0
+                      // CTA issues the MMAs, every CTA drains its own 128 accumulator rows
   const float* bias;
   const __nv_bfloat16* addend;
   int add_tma;        // the addend tile is TMA-loaded into the group's staging tile at the START of the tile's drain (same
@@ -115,10 +108,6 @@ struct IgemmParams {
   const float* gate_h1;
 };
 
-__device__ __forceinline__ uint64_t umma_desc_sw128_bo(uint32_t smem_addr, uint32_t lbo, uint32_t sbo, uint32_t bo) {
-  return umma_desc_sw128(smem_addr, lbo, sbo) | ((uint64_t)(bo & 7u) << 49);
-}
-
 // kPair: the CTA-pair variant is a separate instantiation — a kernel that contains cta_group::2 instructions can only
 // be launched as (multiples of) 2-CTA clusters, so the single-CTA kernel must not contain them.
 template <bool kHasAdd, bool kPair>
@@ -128,8 +117,9 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
                   const __grid_constant__ CUtensorMap tmAdd, const IgemmParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  const int a_slots = p.dm ? 2 : 1;                                    // activation tiles per stage
-  const int nbuf = p.dm ? 4 : 2;                                       // accumulators in TMEM
+  const bool dm = !kPair && p.dm != 0;                                 // pair mode never runs double-M items
+  const int a_slots = dm ? 2 : 1;                                      // activation tiles per stage
+  const int nbuf = dm ? 4 : 2;                                         // accumulators in TMEM
   const int stage_bytes = a_slots * p.a_stage_bytes + (p.wres ? 0 : p.b_stage_bytes);
   const int ctile_bytes = p.ctile_bytes;
   uint8_t* ctile0 = smem + p.stages * stage_bytes;                     // per group: 128 x block_n bf16, 1024 B aligned
@@ -149,32 +139,29 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
   const int lane = threadIdx.x & 31;
   // Work items ("super tiles") are numbered n-fastest: item u = (m-group u / n_tiles, n-tile u % n_tiles); the CTA of
   // rank r in its cluster takes m-tile m-group * cluster + r, cluster q takes items q, q + #clusters, ...
-  const int C = p.cluster;
-  const uint32_t crank = C > 1 ? cluster_ctarank() : 0u;
-  const uint16_t cmask = (uint16_t)((1u << C) - 1u);
+  constexpr int C = kPair ? 2 : 1;                                     // CTAs per cluster
+  const uint32_t crank = kPair ? cluster_ctarank() : 0u;
   const int cluster_id = (int)blockIdx.x / C;
   const int num_clusters = (int)gridDim.x / C;
-  const int per_item = p.dm ? 2 : C;                                   // m-tiles per work item
+  const int per_item = dm ? 2 : C;                                     // m-tiles per work item
   const int total_items = ((p.m_tiles + per_item - 1) / per_item) * p.n_tiles;
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < p.stages; ++s) {
       mbar_init(&full_bar[s], 1);
-      // multicast mode: every CTA of the cluster reads the shared weight slot; pair mode: one (multicast) commit of
-      // the leader's MMAs frees the slot in both CTAs
-      mbar_init(&empty_bar[s], p.pair ? 1u : (uint32_t)C);
+      mbar_init(&empty_bar[s], 1);   // pair mode: one multicast commit of the leader's MMAs frees it in both CTAs
     }
     mbar_init(wres_bar, 1);
     for (int b = 0; b < kMaxEpiGroups; ++b) mbar_init(&add_bar[b], 1);
     for (int b = 0; b < 4; ++b) {
       mbar_init(&tmem_full_bar[b], 1);
-      mbar_init(&tmem_empty_bar[b], p.pair ? 8u : 4u);   // one arrival per epilogue warp (of both CTAs of a pair)
+      mbar_init(&tmem_empty_bar[b], kPair ? 8u : 4u);   // one arrival per epilogue warp (of both CTAs of a pair)
     }
     fence_barrier_init();
     tma_prefetch_desc(&tmA0);
     tma_prefetch_desc(&tmB);
     if (p.cb1 > 0) tma_prefetch_desc(&tmA1);
-    if (p.tma_store) tma_prefetch_desc(&tmY);
+    tma_prefetch_desc(&tmY);
   }
   uint32_t tmem_cols = 32;
   while ((int)tmem_cols < nbuf * p.block_n) tmem_cols <<= 1;
@@ -189,7 +176,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
   }
   tc_fence_before();
   __syncthreads();
-  if (C > 1) cluster_sync_all();       // peers' barriers are initialised before any multicast can reach them
+  if constexpr (kPair) cluster_sync_all();   // the peer's barriers are initialised before anything can signal them
   tc_fence_after();
   // (B200SEG_PDL) everything above — barrier init, descriptor prefetch, TMEM allocation — may overlap the previous
   // kernel's tail; nothing below may run before that kernel has completed
@@ -202,14 +189,13 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
     int stage = 0;
     uint32_t phase = 0;
     // pair mode: the leader's barrier collects the bytes of BOTH CTAs (own A tile + half of B each)
-    const uint32_t tx = (uint32_t)(a_slots * p.a_tx_bytes + (p.wres ? 0 : p.b_stage_bytes)) * (p.pair ? 2u : 1u);
-    const int b_taps = p.halo ? 3 : 1;           // weight taps per stage
-    const int b_rows = p.block_n / C;            // weight rows this CTA fetches (and multicasts) per tap
+    const uint32_t tx = (uint32_t)(a_slots * p.a_tx_bytes + (p.wres ? 0 : p.b_stage_bytes)) * (uint32_t)C;
+    const int b_rows = p.block_n / C;            // weight rows this CTA fetches per tap
     if (p.wres) {
       // weight-resident mode: every weight block the K loop of a tile walks — (phase,) tap group o, channel block cb,
       // in that order, the same boxes the streamed stages use — is fetched once, onto one barrier (n_tiles == 1)
       if (elect_one()) {
-        const uint32_t wtx = (uint32_t)p.wres_bytes * (p.pair ? 2u : 1u);
+        const uint32_t wtx = (uint32_t)p.wres_bytes * (uint32_t)C;
         uint32_t lbar = 0u;
         if constexpr (kPair) {
           lbar = mapa_shared(smem_u32(wres_bar), 0);
@@ -241,7 +227,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
       int w0s[2], h0s[2], n0s[2];
       int tph = 0;                                 // fold == 1: the phase of the item's tile(s)
       for (int q = 0; q < a_slots; ++q) {
-        int t = m_group * per_item + (p.dm ? q : (int)crank);
+        int t = m_group * per_item + (dm ? q : (int)crank);
         if (t >= p.m_tiles) t = p.m_tiles - 1;
         if (p.fold == 1) {
           if (p.fold_il) {
@@ -257,11 +243,11 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
         const int tn_i = fast_div(t1, p.th, p.mg_th);
         const int th_i = t1 - tn_i * p.th;
         w0s[q] = tw_i * p.Wb;
-        h0s[q] = th_i * (p.rp ? 2 : p.Hb);
+        h0s[q] = th_i * p.Hb;
         n0s[q] = tn_i * p.Nb;
       }
       const int w0 = w0s[0], h0 = h0s[0], n0 = n0s[0];
-      const int outer = p.rp ? 4 : (p.halo ? 3 : p.taps);   // halo mode: one iteration per (input row, channel block)
+      const int outer = p.halo ? 3 : p.taps;      // halo mode: one iteration per (input row, channel block)
       for (int o = 0; o < outer; ++o) {
         int dr = 0, ds = 0, tap0 = o;
         int fa = 0, fb = 0;                        // fold == 2: sub-lattice (a, b) of dz this tap reads
@@ -274,10 +260,6 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
           dr = (o >> 1) - (1 - (tph >> 1));
           ds = (o & 1) - (1 - (tph & 1));
           tap0 = tph * 4 + o;
-        } else if (p.rp) {
-          dr = o - 1;
-          ds = -1;
-          tap0 = (o - 1) * 3;          // first tap of the stacked pair (filter rows o-1 and o)
         } else if (p.halo) {
           dr = o - 1;
           ds = -1;
@@ -317,19 +299,8 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
             } else {
             mbar_arrive_expect_tx(&full_bar[stage], tx);
             load_a(sa, w0, h0, n0, 0u);
-            if (p.dm) load_a(sa + p.a_stage_bytes, w0s[1], h0s[1], n0s[1], 0u);   // second tile of the item
-            if (p.wres) {
-              // weights are resident
-            } else if (p.rp) {
-              for (int tp = 0; tp < 3; ++tp)       // [W(o-1, tp) ; W(o, tp)]: 2 taps, element stride 3, 64 rows each
-                tma_load_3d(sb + tp * (128 * 128), &tmB, &full_bar[stage], cb * kKBlock, 0, tap0 + tp);
-            } else if (C == 1) {
-              tma_load_3d(sb, &tmB, &full_bar[stage], cb * kKBlock, n_tile * p.block_n, tap0);
-            } else {
-              for (int tp = 0; tp < b_taps; ++tp)
-                tma_load_3d_mc(sb + (tp * p.block_n + (int)crank * b_rows) * 128, &tmB, &full_bar[stage],
-                               cb * kKBlock, n_tile * p.block_n + (int)crank * b_rows, tap0 + tp, cmask);
-            }
+            if (dm) load_a(sa + p.a_stage_bytes, w0s[1], h0s[1], n0s[1], 0u);   // second tile of the item
+            if (!p.wres) tma_load_3d(sb, &tmB, &full_bar[stage], cb * kKBlock, n_tile * p.block_n, tap0);
             }
             }
           }
@@ -352,7 +323,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
     uint32_t phase = 0;
     int ti = 0;
     const int sub = p.halo ? 3 : 1;
-    const int nb_shift = p.dm ? 2 : 1;           // log2(accumulators in TMEM)
+    const int nb_shift = dm ? 2 : 1;             // log2(accumulators in TMEM)
     const uint32_t wres_addr = smem_u32(wres_base);
     if (p.wres) {
       mbar_wait(wres_bar, 0);                    // the resident weights (of both CTAs of a pair) have landed
@@ -378,54 +349,35 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
           const uint32_t a_addr = smem_u32(smem + stage * stage_bytes);
           const uint32_t b_addr = p.wres ? wres_addr + (uint32_t)((wres_it0 + it) * p.b_stage_bytes)
                                          : a_addr + a_slots * p.a_stage_bytes;
-          if (!p.base_off_mode) {
-            // Descriptors differ only in the 14-bit start-address field (bytes >> 4) of the low word, and smem
-            // addresses are < 256 KB, so stepping a descriptor is one 32-bit add: +2 per 16-element K step (32 B),
-            // +8 per pixel of halo shift (128 B), +8 * BLOCK_N per weight tap.  This keeps the single issuing thread
-            // at a few instructions per MMA — it paces the N <= 128 tiles otherwise.
-            const int nsub = (p.debug_skip & 2) ? 0 : sub;
-            for (int q = 0; q < a_slots; ++q) {
-              const uint32_t lt = (uint32_t)(a_slots * ti + q);
-              const uint32_t d_tmem = tmem_base + (lt & (uint32_t)(nbuf - 1)) * (uint32_t)p.block_n;
-              uint32_t a_lo = desc_lo0 + ((a_addr + (uint32_t)(q * p.a_stage_bytes)) >> 4);
-              uint32_t b_lo = desc_lo0 + (b_addr >> 4);
-              for (int s = 0; s < nsub; ++s) {     // (a fully unrolled 12-MMA variant measured slower)
-                if constexpr (kPair) {
+          // Descriptors differ only in the 14-bit start-address field (bytes >> 4) of the low word, and smem
+          // addresses are < 256 KB, so stepping a descriptor is one 32-bit add: +2 per 16-element K step (32 B),
+          // +8 per pixel of halo shift (128 B), +8 * BLOCK_N per weight tap.  This keeps the single issuing thread
+          // at a few instructions per MMA — it paces the N <= 128 tiles otherwise.
+          const int nsub = (p.debug_skip & 2) ? 0 : sub;
+          for (int q = 0; q < a_slots; ++q) {
+            const uint32_t lt = (uint32_t)(a_slots * ti + q);
+            const uint32_t d_tmem = tmem_base + (lt & (uint32_t)(nbuf - 1)) * (uint32_t)p.block_n;
+            uint32_t a_lo = desc_lo0 + ((a_addr + (uint32_t)(q * p.a_stage_bytes)) >> 4);
+            uint32_t b_lo = desc_lo0 + (b_addr >> 4);
+            for (int s = 0; s < nsub; ++s) {     // (a fully unrolled 12-MMA variant measured slower)
+              if constexpr (kPair) {
 #pragma unroll
-                  for (int k = 0; k < kKBlock / 16; ++k)
-                    umma_bf16_pair(d_tmem, desc_hi | (uint64_t)(a_lo + 2 * k), desc_hi | (uint64_t)(b_lo + 2 * k), idesc,
-                                   (it | s | k) != 0 ? 1u : 0u);
-                } else {
+                for (int k = 0; k < kKBlock / 16; ++k)
+                  umma_bf16_pair(d_tmem, desc_hi | (uint64_t)(a_lo + 2 * k), desc_hi | (uint64_t)(b_lo + 2 * k), idesc,
+                                 (it | s | k) != 0 ? 1u : 0u);
+              } else {
 #pragma unroll
-                  for (int k = 0; k < kKBlock / 16; ++k)
-                    umma_bf16(d_tmem, desc_hi | (uint64_t)(a_lo + 2 * k), desc_hi | (uint64_t)(b_lo + 2 * k), idesc,
-                              (it | s | k) != 0 ? 1u : 0u);
-                }
-                a_lo += 8;
-                b_lo += b_tap_step;
+                for (int k = 0; k < kKBlock / 16; ++k)
+                  umma_bf16(d_tmem, desc_hi | (uint64_t)(a_lo + 2 * k), desc_hi | (uint64_t)(b_lo + 2 * k), idesc,
+                            (it | s | k) != 0 ? 1u : 0u);
               }
-            }
-          } else {
-          const uint32_t d_tmem = tmem_base + (uint32_t)((ti & 1) * p.block_n);
-          for (int s = 0; s < ((p.debug_skip & 2) ? 0 : sub); ++s) {
-            const uint32_t a_s = a_addr + s * 128;            // halo mode: shift by s pixels (rows of 128 B)
-            const uint32_t b_s = b_addr + s * p.block_n * 128;
-            const uint32_t bo = p.base_off_mode ? ((a_s >> 7) & 7u) : 0u;
-#pragma unroll
-            for (int k = 0; k < kKBlock / 16; ++k) {
-              const uint64_t da = umma_desc_sw128_bo(a_s + k * 32, 16, 1024, bo);
-              const uint64_t db = umma_desc_sw128(b_s + k * 32, 16, 1024);
-              umma_bf16(d_tmem, da, db, idesc, (it | s | k) != 0 ? 1u : 0u);
+              a_lo += 8;
+              b_lo += b_tap_step;
             }
           }
-          }
-          // frees this smem slot (in every CTA that multicasts into it) when the MMAs have read it
-          if constexpr (kPair) {
-            umma_commit_pair(&empty_bar[stage], 3);
-          } else {
-            if (C == 1) umma_commit(&empty_bar[stage]);
-            else umma_commit_mc(&empty_bar[stage], cmask);
-          }
+          // frees this smem slot (in both CTAs of a pair) when the MMAs have read it
+          if constexpr (kPair) umma_commit_pair(&empty_bar[stage], 3);
+          else umma_commit(&empty_bar[stage]);
         }
         __syncwarp();
         if (++stage == p.stages) {
@@ -473,7 +425,6 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
     for (int i = 0; i < 16; ++i) acc[i] = 0.0;
     // fp32 partial sums of the last few tiles (32 values each, as many as one N = 256 tile contributes): the fp64 pipe
     // is narrow, so the conversion + DADD per channel runs once per 32 rows instead of once per tile
-    const int fold_tiles = 32 / nchunks;         // 8, 4, 2, 1 tiles for N = 32, 64, 128, 256
     float fs[8], fq[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) fs[j] = fq[j] = 0.f;
@@ -496,7 +447,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
 #pragma unroll
         for (int i = 0; i < 16; ++i) acc[i] += __shfl_xor_sync(0xffffffffu, acc[i], off);
       }
-      if (p.tma_store && et == 0) tma_store_wait_read();
+      if (et == 0) tma_store_wait_read();
       asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");    // staging tile is free
       double* red = reinterpret_cast<double*>(ctile);                 // [warp][sum | sumsq][block_n]
       if (lane < nchunks) {
@@ -513,7 +464,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
         double v = 0.0;
 #pragma unroll
         for (int w = 0; w < 4; ++w) v += red[(w * 2 + which) * p.block_n + c];
-        const int sidx = which * p.cout + n_tile_ * p.block_n + (p.rp ? (c & 63) : c);
+        const int sidx = which * p.cout + n_tile_ * p.block_n + c;
         if (p.stats_partial != nullptr)      // this thread owns slot sidx of this (CTA, group) row for the whole launch
           p.stats_partial[(size_t)(blockIdx.x * p.epi_groups + g) * (2 * p.cout) + sidx] += v;
         else
@@ -526,15 +477,15 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
 
     int cur_n_tile = -1;
     uint32_t add_phase = 0;                      // parity of this group's addend barrier
-    const int nb_shift = p.dm ? 2 : 1;           // log2(accumulators in TMEM)
+    const int nb_shift = dm ? 2 : 1;             // log2(accumulators in TMEM)
     // ti = local tile counter of this CTA (group g takes ti = g, g + G, ...); double-M: item = ti / 2, tile ti & 1
     for (int ti = g;; ti += G) {
-      const int item = cluster_id + (p.dm ? (ti >> 1) : ti) * num_clusters;
+      const int item = cluster_id + (dm ? (ti >> 1) : ti) * num_clusters;
       if (item >= total_items) break;
       const int m_group = fast_div(item, p.n_tiles, p.mg_nt);
       const int n_tile = item - m_group * p.n_tiles;
       const int ch_base = n_tile * p.block_n;
-      int t = m_group * per_item + (p.dm ? (ti & 1) : (int)crank);
+      int t = m_group * per_item + (dm ? (ti & 1) : (int)crank);
       int eph = 0;                                 // fold == 1: phase of this tile
       if (p.fold == 1 && t < p.m_tiles) {
         eph = p.fold_il ? ((t >> 1) & 3) : fast_div(t, p.m_tiles_phase, p.mg_mtp);
@@ -557,7 +508,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
         if (cur_n_tile >= 0 && p.stats != nullptr) flush_stats(cur_n_tile);
         asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");   // everyone is done reading the old bias slice
         for (int i = et; i < p.block_n; i += 128) {
-          s_bias[i] = p.bias ? p.bias[ch_base + (p.rp ? (i & 63) : i)] : 0.f;
+          s_bias[i] = p.bias ? p.bias[ch_base + i] : 0.f;
           if (p.gate_x != nullptr) s_psi[i] = p.gate_wpsi[i];
         }
         cur_n_tile = n_tile;
@@ -567,17 +518,17 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
       const int tw_i = t - t1 * p.tw;
       const int tn_i = fast_div(t1, p.th, p.mg_th);
       const int th_i = t1 - tn_i * p.th;
-      const int w0 = tw_i * p.Wb, h0 = th_i * (p.rp ? 2 : p.Hb), n0 = tn_i * p.Nb;
+      const int w0 = tw_i * p.Wb, h0 = th_i * p.Hb, n0 = tn_i * p.Nb;
       // pixels of the tile that exist (tiles at the right / bottom / batch edge are clipped): row r of the tile is pixel
       // (n0 + r / (Wb Hb), h0 + (r / Wb) % Hb, w0 + r % Wb); all three box extents are powers of two
-      const bool tile_full = w0 + p.Wb <= p.W && h0 + (p.rp ? 2 : p.Hb) <= p.H && n0 + p.Nb <= p.N;
+      const bool tile_full = w0 + p.Wb <= p.W && h0 + p.Hb <= p.H && n0 + p.Nb <= p.N;
       auto row_valid = [&](int r) {
         return tile_full || (w0 + r % p.Wb < p.W && h0 + (r / p.Wb) % p.Hb < p.H && n0 + r / (p.Wb * p.Hb) < p.N);
       };
       const int buf = ti & (nbuf - 1);
 
       // the group's previous TMA store must have finished READING the staging tile before it is overwritten
-      if (p.tma_store && et == 0) tma_store_wait_read();
+      if (et == 0) tma_store_wait_read();
       asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");
       if (kHasAdd && p.add_tma) {
         // the addend tile lands in the staging tile while this group waits for the accumulator
@@ -603,13 +554,13 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
         // addend ran at 3.7 TB/s where the same launch without addend reaches 5 TB/s).  Pull the rows of the NEXT tile
         // this group will drain into L2 now; its loads then hit L2.
         const int ti2 = ti + G;
-        const int item2 = cluster_id + (p.dm ? (ti2 >> 1) : ti2) * num_clusters;
+        const int item2 = cluster_id + (dm ? (ti2 >> 1) : ti2) * num_clusters;
         if (p.add_tma) {
           mbar_wait(&add_bar[g], add_phase);
           add_phase ^= 1u;
-        } else if (item2 < total_items && !p.rp) {
+        } else if (item2 < total_items) {
           const int m_group2 = fast_div(item2, p.n_tiles, p.mg_nt);
-          const int t2 = m_group2 * per_item + (p.dm ? (ti2 & 1) : (int)crank);
+          const int t2 = m_group2 * per_item + (dm ? (ti2 & 1) : (int)crank);
           if (t2 < p.m_tiles) {
             const int u1 = fast_div(t2, p.tw, p.mg_tw);
             const int u_w = t2 - u1 * p.tw;
@@ -741,34 +692,18 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
       fence_proxy_async();                       // generic-proxy smem writes -> visible to the TMA store
       asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");
 
-      if (p.tma_store) {
-        if (et == 0) {
-          if (p.rp) {                 // panel 0 = output row h0 + 1, panel 1 = output row h0
-            tma_store_4d(&tmY, ctile, 0, w0, h0 + 1, n0);
-            tma_store_4d(&tmY, ctile + kTileM * 128, 0, w0, h0, n0);
-          } else if (p.fold == 1) {    // phase (a, b) of the fine grid: 5-D view (b*C + c, w, a, h, n)
-            for (int pn = 0; pn < (p.block_n >> 6); ++pn)
-              tma_store_5d(&tmY, ctile + pn * (kTileM * 128), (eph & 1) * p.fold_c + ch_base + pn * 64, w0, eph >> 1, h0,
-                           n0);
-          } else if (p.block_n >= 64) {
-            for (int pn = 0; pn < (p.block_n >> 6); ++pn)
-              tma_store_4d(&tmY, ctile + pn * (kTileM * 128), ch_base + pn * 64, w0, h0, n0);
-          } else {
-            tma_store_4d(&tmY, ctile, ch_base, w0, h0, n0);     // 32-channel tile: 64 B rows, 64B-swizzle map
-          }
-          tma_store_commit();
+      if (et == 0) {
+        if (p.fold == 1) {          // phase (a, b) of the fine grid: 5-D view (b*C + c, w, a, h, n)
+          for (int pn = 0; pn < (p.block_n >> 6); ++pn)
+            tma_store_5d(&tmY, ctile + pn * (kTileM * 128), (eph & 1) * p.fold_c + ch_base + pn * 64, w0, eph >> 1, h0,
+                         n0);
+        } else if (p.block_n >= 64) {
+          for (int pn = 0; pn < (p.block_n >> 6); ++pn)
+            tma_store_4d(&tmY, ctile + pn * (kTileM * 128), ch_base + pn * 64, w0, h0, n0);
+        } else {
+          tma_store_4d(&tmY, ctile, ch_base, w0, h0, n0);     // 32-channel tile: 64 B rows, 64B-swizzle map
         }
-      } else {
-        // coalesced copy-out: consecutive threads write consecutive 16 B of consecutive pixels
-        for (int idx = et; idx < kTileM * nchunks; idx += 128) {
-          const int r = idx / nchunks, ck = idx % nchunks;
-          if (row_valid(r)) {
-            const int rwl = r % p.Wb, rhl = (r / p.Wb) % p.Hb, rnl = r / (p.Wb * p.Hb);
-            const long long ro = (n0 + rnl) * p.y_sn + (h0 + rhl) * p.y_sh + (w0 + rwl) * p.y_sw;
-            const uint4 u = *reinterpret_cast<const uint4*>(ctile + ctile_off(p.block_n, r, ck * 8));
-            *reinterpret_cast<uint4*>(p.y + ro + ch_base + ck * 8) = u;
-          }
-        }
+        tma_store_commit();
       }
       if (p.stats != nullptr) {
         // column sums of the ROUNDED outputs (what BatchNorm sees under autocast), 8 channels per thread: rows
@@ -803,16 +738,16 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
             stats_accum(*reinterpret_cast<const uint4*>(ctile + ctile_off(p.block_n, r, schunk * 8)), fs, fq);
           }
         }
-        if (++fpending >= fold_tiles) fold_stats();
+        if (++fpending * nchunks >= 32) fold_stats();   // every 8, 4, 2, 1 tiles for N = 32, 64, 128, 256
       }
     }
     if (p.stats != nullptr && cur_n_tile >= 0) flush_stats(cur_n_tile);
-    if (p.tma_store && et == 0) tma_store_wait_all();
+    if (et == 0) tma_store_wait_all();
   }
 
   tc_fence_before();
   __syncthreads();
-  if (C > 1) cluster_sync_all();       // no CTA leaves while a peer may still signal its barriers
+  if constexpr (kPair) cluster_sync_all();   // no CTA leaves while its peer may still signal its barriers
   if (warp == 1) {
     if constexpr (kPair) tmem_dealloc_pair(tmem_base, tmem_cols);
     else tmem_dealloc(tmem_base, tmem_cols);
@@ -946,43 +881,21 @@ static int conv_igemm_launch(const b2_conv_args* a, cudaStream_t stream, const G
   }
   p.n_tiles = a->cout / p.block_n;
   p.m_tiles_phase = p.m_tiles;
-  p.fold_il = (fold == 1 && p.m_tiles % 2 == 0 && env_int("B200SEG_FOLD_INTERLEAVE", 1) != 0 &&
-               env_int("B200SEG_CLUSTER", 0) <= 2) ? 1 : 0;
+  p.fold_il = (fold == 1 && p.m_tiles % 2 == 0) ? 1 : 0;
   if (fold == 1) p.m_tiles *= 4;                 // the four phases are an extra tile dimension
-  p.y = static_cast<__nv_bfloat16*>(a->y);
-  p.ldy = a->ldy;
   p.bias = a->bias;
   p.addend = static_cast<const __nv_bfloat16*>(a->addend);
   p.ldadd = a->ldadd;
   p.stats = a->stats;
   p.relu = a->relu;
   p.add_after_act = (a->addend != nullptr && a->add_after_act) ? 1 : 0;
-  // halo mode: 3x3, tile == one row segment of 128 pixels
-  const int halo_env = env_int("B200SEG_HALO", 1);
   p.stride = stride;
   p.ksize = a->ksize;
   p.pad_h = a->custom_pad ? a->pad_h : (a->ksize == 3 ? 1 : 0);
   p.pad_w = a->custom_pad ? a->pad_w : (a->ksize == 3 ? 1 : 0);
-  p.halo = (halo_env != 0 && p.taps == 9 && stride == 1 && !a->custom_pad && p.Hb == 1 && p.Nb == 1 &&
-            p.Wb == kTileM) ? 1 : 0;
-  p.base_off_mode = (halo_env == 2) ? 1 : 0;
-  p.tma_store = env_int("B200SEG_TMA_STORE", 1) != 0 ? 1 : 0;
-  p.rp = (p.halo && a->cout == 64 && p.block_n == 64 && a->h % 2 == 0 && a->addend == nullptr && out_mul == 1 &&
-          in_mul == 1 && p.tma_store && env_int("B200SEG_FPROP_ROWPAIR", 0) != 0 &&
-          !(a->stats != nullptr && det_enabled())) ? 1 : 0;   // opt-in, see below (two columns share a statistics slot)
-  // Row-pair mode is parity-tested but off by default: it makes the Cout = 64 MMAs N = 128 (isolated: 64->64 @256^2
-  // 0.390 -> 0.366 ms, 128->64 0.711 -> 0.680 ms) but streams 192 KB of stacked weights per tile pair from L2, and
-  // inside the training step, where the side-stream weight gradients load the same fabric, the gain vanishes.
-  if (p.rp) {
-    p.block_n = 128;                       // two 64-channel panels = two output rows
-    p.n_tiles = 1;
-    p.th = a->h / 2;
-    p.m_tiles = p.tw * p.th * tn;
-    p.a_tx_bytes = (kTileM + 2) * 128;
-    p.a_stage_bytes = ((p.a_tx_bytes + 1023) / 1024) * 1024;
-    p.b_stage_bytes = 3 * 128 * 128;
-    p.num_k_iters = 4 * cbt;
-  } else if (p.halo) {
+  // halo mode: 3x3, tile == one row segment of 128 pixels
+  p.halo = (p.taps == 9 && stride == 1 && !a->custom_pad && p.Hb == 1 && p.Nb == 1 && p.Wb == kTileM) ? 1 : 0;
+  if (p.halo) {
     p.a_tx_bytes = (kTileM + 2) * 128;
     p.a_stage_bytes = ((p.a_tx_bytes + 1023) / 1024) * 1024;
     p.b_stage_bytes = 3 * p.block_n * 128;
@@ -995,7 +908,7 @@ static int conv_igemm_launch(const b2_conv_args* a, cudaStream_t stream, const G
   }
   int ctile_bytes = kTileM * p.block_n * 2;
   if (gate != nullptr) {
-    B2_REQUIRE(p.n_tiles == 1 && !p.rp && out_mul == 1 && in_mul == 1 && stride == 1 && a->ksize == 1 && p.tma_store,
+    B2_REQUIRE(p.n_tiles == 1 && out_mul == 1 && in_mul == 1 && stride == 1 && a->ksize == 1,
                B2_ERR_SHAPE, "fused gate: F_int=%d must be one tile (32 | 64 | 128 | 256) of a plain 1x1 GEMM", a->cout);
     B2_REQUIRE(gate->c % 64 == 0 && gate->ldx % 8 == 0 && (reinterpret_cast<uintptr_t>(gate->x) & 15) == 0, B2_ERR_SHAPE,
                "fused gate: C=%d must be a multiple of 64, x 16 B aligned", gate->c);
@@ -1026,15 +939,14 @@ static int conv_igemm_launch(const b2_conv_args* a, cudaStream_t stream, const G
   // 2 (default) every eligible layer (replaces double-M there).  Measured at batch 64 (profiles/r02_conv_layers_pair*):
   // N = 256 layers 1224 -> 1460 ... 1385 -> 1637 TFLOP/s, 64 -> 128 @128^2 944 -> 1218, 64 -> 64 @256^2 853 -> 910;
   // conv_igemm time inside the training step 16.3 -> 14.7 ms.
+  p.debug_skip = env_int("B200SEG_DEBUG_SKIP", 0);
   {
     const int want = env_int("B200SEG_PAIR", 2);
     p.pair = 0;
-    if (want != 0 && !p.rp && p.m_tiles >= 2 && p.block_n % 16 == 0 && (want >= 2 || p.block_n == 256) &&
-        !(fold == 1 && p.m_tiles_phase % 2 != 0) &&
-        env_int("B200SEG_CLUSTER", 0) <= 1 && env_int("B200SEG_DEBUG_SKIP", 0) == 0) {
+    if (want != 0 && p.m_tiles >= 2 && p.block_n % 16 == 0 && (want >= 2 || p.block_n == 256) &&
+        !(fold == 1 && p.m_tiles_phase % 2 != 0) && p.debug_skip == 0) {
       p.pair = 1;
       p.dm = 0;
-      p.base_off_mode = 0;
       p.b_stage_bytes /= 2;          // each CTA of the pair stages half of the weight rows
     }
   }
@@ -1055,33 +967,16 @@ static int conv_igemm_launch(const b2_conv_args* a, cudaStream_t stream, const G
     // group's drain overlap buys (128->256 @64^2 fprop: 0.164 ms with two groups, 0.125 ms with one)
     if (p.epi_groups == 2 && p.pair && p.block_n == 256 && forced_g == 0 && budget2 / stage_bytes < 4) p.epi_groups = 1;
   }
-  // Clusters: per tile a CTA streams A_bytes + B_bytes / cluster from L2; at about 42 B/clk per SM (L2 -> SM fabric,
-  // 6300 B/clk chip-wide) the weight re-fetch is what bounds every layer with BLOCK_N <= 128.
-  {
-    const double a_bytes = (double)p.a_tx_bytes * p.num_k_iters, b_bytes = (double)p.b_stage_bytes * p.num_k_iters;
-    const double mma_clk = (double)p.num_k_iters * (p.halo ? 3 : 1) * (kKBlock / 16) * (p.block_n / 2);
-    // Measured on B200: no gain at cluster sizes 2 and 4 (the multicast does not relieve what bounds these tiles),
-    // so clusters are opt-in (B200SEG_CLUSTER=2|4) and the default is 1.
-    (void)a_bytes; (void)b_bytes; (void)mma_clk;
-    int c = 1;
-    p.debug_skip = env_int("B200SEG_DEBUG_SKIP", 0);
-    const int forced_c = env_int("B200SEG_CLUSTER", 0);
-    if (forced_c == 1 || forced_c == 2 || forced_c == 4) c = forced_c;
-    while (c > 1 && ((p.block_n / c) % 8 != 0 || p.m_tiles < c)) c /= 2;
-    if (p.rp || p.dm) c = 1;
-    if (p.pair) c = 2;
-    p.cluster = c;
-  }
   // Weight-resident mode (IgemmParams::wres): one n-tile, the whole slab next to >= 4 activation-only stages, and
-  // enough tiles per CTA that fetching all weights before the first MMA costs nothing.  B200SEG_WRES=0 switches it off.
+  // enough tiles per CTA that fetching all weights before the first MMA costs nothing.
   int budget = 232448 - 1024 - tail_bytes - p.epi_groups * ctile_bytes;
   p.wres = 0;
   p.wres_bytes = 0;
   {
     const long long wb = (long long)(fold == 1 ? 4 : 1) * p.num_k_iters * p.b_stage_bytes;
     const int a_only = (p.dm ? 2 : 1) * p.a_stage_bytes;
-    if (env_int("B200SEG_WRES", 1) != 0 && p.n_tiles == 1 && !p.rp && (p.cluster == 1 || p.pair) && !p.base_off_mode &&
-        p.debug_skip == 0 && p.m_tiles >= 4 * num_sms() && wb % 1024 == 0 && (budget - wb) / a_only >= 4) {
+    if (p.n_tiles == 1 && p.debug_skip == 0 && p.m_tiles >= 4 * num_sms() && wb % 1024 == 0 &&
+        (budget - wb) / a_only >= 4) {
       p.wres = 1;
       p.wres_bytes = (int)wb;
       stage_bytes = a_only;
@@ -1127,55 +1022,39 @@ static int conv_igemm_launch(const b2_conv_args* a, cudaStream_t stream, const G
   {
     uint64_t dims[3] = {(uint64_t)(a->c0 + a->c1), (uint64_t)a->cout, (uint64_t)(fold == 1 ? 16 : p.taps)};
     uint64_t str[3] = {2, (uint64_t)a->ktot * 2, (uint64_t)a->w_tap_stride * 2};
-    uint32_t box[3] = {64, (uint32_t)p.block_n, p.halo ? 3u : 1u};
-    if (p.pair) {                 // this CTA's half of the rows, all taps of the stage in one box
-      box[1] = (uint32_t)(p.block_n / 2);
-    } else if (p.cluster > 1) {   // one multicast box per tap: this CTA's share of the rows
-      box[1] = (uint32_t)(p.block_n / p.cluster);
-      box[2] = 1u;
-    }
-    if (p.rp) {                   // two taps three apart (filter rows r and r+1 of one column): traversal stride 3
-      uint32_t box_rp[3] = {64, 64, 6};
-      uint32_t est_rp[3] = {1, 1, 3};
-      rc = encode_tmap_bf16(&tmB, a->wpk, 3, dims, str, box_rp, CU_TENSOR_MAP_SWIZZLE_128B, est_rp);
-    } else {
-      rc = encode_tmap_bf16(&tmB, a->wpk, 3, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B);
-    }
+    // all taps of the stage in one box; pair mode: this CTA's half of the rows
+    uint32_t box[3] = {64, (uint32_t)(p.pair ? p.block_n / 2 : p.block_n), p.halo ? 3u : 1u};
+    rc = encode_tmap_bf16(&tmB, a->wpk, 3, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B);
     if (rc) return rc;
   }
   // output pixel grid (possibly a strided sub-lattice of a larger image: ConvTranspose pixel shuffle)
   const long long ow = (long long)a->w * out_mul, oh = (long long)a->h * out_mul;
-  p.y_sw = (long long)out_mul * a->ldy;
-  p.y_sh = (long long)out_mul * ow * a->ldy;
-  p.y_sn = oh * ow * a->ldy;
-  p.y = static_cast<__nv_bfloat16*>(a->y) + ((long long)a->out_off_h * ow + a->out_off_w) * a->ldy;
-  if (p.tma_store) {
-    if (fold == 1) {              // y [n, 2h, 2w, Cout] as (b*C + c, w, a, h, n)
-      B2_REQUIRE(p.block_n >= 64, B2_ERR_SHAPE, "merged UpConv fprop needs cout >= 64");
-      const uint64_t Cc = (uint64_t)a->cout, W2 = (uint64_t)a->w, H2 = (uint64_t)a->h;
-      uint64_t dims[5] = {2 * Cc, W2, 2, H2, (uint64_t)a->n};
-      uint64_t str[5] = {2, 2 * Cc * 2, 2 * W2 * Cc * 2, 4 * W2 * Cc * 2, 4 * H2 * W2 * Cc * 2};
-      uint32_t box[5] = {64, (uint32_t)p.Wb, 1, (uint32_t)p.Hb, (uint32_t)p.Nb};
-      rc = encode_tmap_bf16(&tmY, a->y, 5, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B);
-    } else if (gate != nullptr) { // the gate's output has C channels (64-channel boxes), not F_int
-      rc = encode_act_tmap_ex(&tmY, p.y, gate->c, a->n, a->h, a->w, p.y_sw, p.y_sh, p.y_sn, p.Wb, p.Hb, p.Nb, 1);
-    } else if (p.block_n >= 64) {
-      rc = encode_act_tmap_ex(&tmY, p.y, a->cout, a->n, a->h, a->w, p.y_sw, p.y_sh, p.y_sn, p.Wb, p.Hb, p.Nb, 1);
-    } else {
-      // 32-channel tiles are staged as 64 B rows with chunk ^= (row >> 1) & 3 == TMA's 64B swizzle
-      uint64_t dims[4] = {(uint64_t)a->cout, (uint64_t)a->w, (uint64_t)a->h, (uint64_t)a->n};
-      uint64_t str[4] = {2, (uint64_t)p.y_sw * 2, (uint64_t)p.y_sh * 2, (uint64_t)p.y_sn * 2};
-      uint32_t box[4] = {32, (uint32_t)p.Wb, (uint32_t)p.Hb, (uint32_t)p.Nb};
-      rc = encode_tmap_bf16(&tmY, p.y, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B);
-    }
-    if (rc) return rc;
+  const long long y_sw = (long long)out_mul * a->ldy;      // element strides of the output pixel grid
+  const long long y_sh = (long long)out_mul * ow * a->ldy;
+  const long long y_sn = oh * ow * a->ldy;
+  void* y = static_cast<__nv_bfloat16*>(a->y) + ((long long)a->out_off_h * ow + a->out_off_w) * a->ldy;
+  if (fold == 1) {                // y [n, 2h, 2w, Cout] as (b*C + c, w, a, h, n)
+    B2_REQUIRE(p.block_n >= 64, B2_ERR_SHAPE, "merged UpConv fprop needs cout >= 64");
+    const uint64_t Cc = (uint64_t)a->cout, W2 = (uint64_t)a->w, H2 = (uint64_t)a->h;
+    uint64_t dims[5] = {2 * Cc, W2, 2, H2, (uint64_t)a->n};
+    uint64_t str[5] = {2, 2 * Cc * 2, 2 * W2 * Cc * 2, 4 * W2 * Cc * 2, 4 * H2 * W2 * Cc * 2};
+    uint32_t box[5] = {64, (uint32_t)p.Wb, 1, (uint32_t)p.Hb, (uint32_t)p.Nb};
+    rc = encode_tmap_bf16(&tmY, a->y, 5, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B);
+  } else if (gate != nullptr) {   // the gate's output has C channels (64-channel boxes), not F_int
+    rc = encode_act_tmap_ex(&tmY, y, gate->c, a->n, a->h, a->w, y_sw, y_sh, y_sn, p.Wb, p.Hb, p.Nb, 1);
+  } else if (p.block_n >= 64) {
+    rc = encode_act_tmap_ex(&tmY, y, a->cout, a->n, a->h, a->w, y_sw, y_sh, y_sn, p.Wb, p.Hb, p.Nb, 1);
   } else {
-    tmY = tmA0;
+    // 32-channel tiles are staged as 64 B rows with chunk ^= (row >> 1) & 3 == TMA's 64B swizzle
+    uint64_t dims[4] = {(uint64_t)a->cout, (uint64_t)a->w, (uint64_t)a->h, (uint64_t)a->n};
+    uint64_t str[4] = {2, (uint64_t)y_sw * 2, (uint64_t)y_sh * 2, (uint64_t)y_sn * 2};
+    uint32_t box[4] = {32, (uint32_t)p.Wb, (uint32_t)p.Hb, (uint32_t)p.Nb};
+    rc = encode_tmap_bf16(&tmY, y, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B);
   }
+  if (rc) return rc;
   CUtensorMap tmAdd = tmY;
   p.add_tma = 0;
-  if (a->addend != nullptr && p.tma_store && p.block_n >= 64 && fold == 0 && gate == nullptr && !p.rp && out_mul == 1 &&
-      a->cout % 64 == 0 && env_int("B200SEG_ADD_TMA", 1) != 0) {
+  if (a->addend != nullptr && p.block_n >= 64 && fold == 0 && gate == nullptr && out_mul == 1 && a->cout % 64 == 0) {
     rc = encode_act_tmap_ex(&tmAdd, a->addend, a->cout, a->n, a->h, a->w, a->ldadd, (long long)a->ldadd * a->w,
                             (long long)a->ldadd * a->w * a->h, p.Wb, p.Hb, p.Nb, 1);
     if (rc) return rc;
@@ -1196,30 +1075,30 @@ static int conv_igemm_launch(const b2_conv_args* a, cudaStream_t stream, const G
   }
   // persistent grid: one CTA per SM.  When the number of clusters is a multiple of n_tiles every CTA keeps one n-tile
   // for its whole life and its BN statistics stay in registers; otherwise they are flushed whenever the slab changes.
-  const int C = p.cluster;
+  const int C = p.pair ? 2 : 1;        // CTAs per cluster: pair mode launches 2-CTA clusters
   int clusters = num_sms() / C;
-  if (C > 1) {
+  if (p.pair) {
     static std::mutex mc_mu;
-    static int max_clusters[5] = {0, 0, 0, 0, 0};
+    static int max_pairs = 0;
     std::lock_guard<std::mutex> mc_lock(mc_mu);
-    if (max_clusters[C] == 0) {
+    if (max_pairs == 0) {
       cudaLaunchConfig_t qc = {};
-      qc.gridDim = dim3((unsigned)(num_sms() / C * C));
+      qc.gridDim = dim3((unsigned)(num_sms() / 2 * 2));
       qc.blockDim = dim3(kThreads);
       qc.dynamicSmemBytes = 232448;
       cudaLaunchAttribute qa[1];
       qa[0].id = cudaLaunchAttributeClusterDimension;
-      qa[0].val.clusterDim.x = (unsigned)C;
+      qa[0].val.clusterDim.x = 2;
       qa[0].val.clusterDim.y = 1;
       qa[0].val.clusterDim.z = 1;
       qc.attrs = qa;
       qc.numAttrs = 1;
       int n = 0;
       B2_CHECK_CUDA(cudaOccupancyMaxActiveClusters(&n, conv_igemm_kernel<false, false>, &qc));
-      B2_REQUIRE(n > 0, B2_ERR_CUDA, "no cluster of %d CTAs can be resident", C);
-      max_clusters[C] = n;
+      B2_REQUIRE(n > 0, B2_ERR_CUDA, "no cluster of 2 CTAs can be resident");
+      max_pairs = n;
     }
-    if (clusters > max_clusters[C]) clusters = max_clusters[C];
+    if (clusters > max_pairs) clusters = max_pairs;
   }
   const int per_item = p.dm ? 2 : C;
   const long long total = (long long)((p.m_tiles + per_item - 1) / per_item) * p.n_tiles;
@@ -1245,7 +1124,6 @@ static int conv_igemm_launch(const b2_conv_args* a, cudaStream_t stream, const G
   }
   if (clusters > total) clusters = (int)total;
   if (clusters > p.n_tiles && (total / clusters) >= 16) clusters = (clusters / p.n_tiles) * p.n_tiles;
-  p.m_stride = 0;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)(clusters * C));
   cfg.blockDim = dim3(kThreads);

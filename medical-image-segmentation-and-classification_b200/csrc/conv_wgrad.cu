@@ -65,12 +65,6 @@ struct WgradParams {
                      // the box (the 128B swizzle is a function of the absolute smem address).  Halves the bytes a
                      // CTA pulls through the L2 -> SM fabric.  nbox = boxes per stage (2), kXhBox bytes apart.
   int nbox;
-  int tapn;          // X-halo mode, single CTA: the three taps of one halo box are ONE N = 192 MMA — N blocks one pixel
-                     // (128 B) apart, i.e. a descriptor with LBO = 128 B over the overlapping shifted views — instead of
-                     // three N = 128 MMAs over both boxes: the dY slice is read twice instead of three times per K step
-                     // (the kernel is bound by shared-memory operand bandwidth).  Accumulators [box][tap][64].
-                     // MEASURED SLOWER (B200SEG_WG_TAPN=1, off by default): 64->64 @256^2 0.339 -> 0.372 ms, 128->128
-                     // @128^2 0.259 -> 0.288 ms — the overlapping N blocks cost more than the saved dY reads.
   int pair;          // CTA pair (cta_group::2): blockIdx.x = rank + 2 * (rg + gy * (co pair + co pairs * channel group))
   int fold;          // merged folded-UpConv weight gradient (b2_wgrad_args::fold): dY is the FINE tensor, phase (a, b) its
                      // (2h+a, 2w+b) sub-lattice; a CTA owns (a, filter row ty) = blockIdx % 4, loads the b = 0 and b = 1
@@ -150,9 +144,10 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmDY, const __grid_constan
   // number of live column blocks for this CTA (1x1 groups may run past the last channel block)
   int live_cb = p.cpb;
   if (cib_base + live_cb > cbt) live_cb = cbt - cib_base;
+  const int rowpair = kPair ? 0 : p.rowpair;                    // pair mode never runs row pairs
   const int grp_cols = live_cb * p.ksize;                       // columns per X-row group (row-pair mode)
-  const int ncol_live = p.rowpair ? p.rowpair * grp_cols : grp_cols;
-  const int xh_live = p.rowpair ? p.rowpair : live_cb;           // X-halo mode: boxes this CTA fills per stage
+  const int ncol_live = rowpair ? rowpair * grp_cols : grp_cols;
+  const int xh_live = rowpair ? rowpair : live_cb;              // X-halo mode: boxes this CTA fills per stage
 
   if (warp == 0) {
     // TMA producer: warp-uniform loop, one elected lane issues; chunk coordinates advance incrementally
@@ -214,7 +209,7 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmDY, const __grid_constan
           } else {
           mbar_arrive_expect_tx(&full_bar[stage], tx);
           // dY: both 64-channel blocks of the 128-row M tile in one 5-D box (.., channel block)
-          if (p.rowpair) {     // dY rows h0 and h0 + 1 (zero fill below the image)
+          if (rowpair) {       // dY rows h0 and h0 + 1 (zero fill below the image)
             tma_load_4d(sa, &tmDY, &full_bar[stage], 0, w0, h0, n0);
             tma_load_4d(sa + kBoxBytes, &tmDY, &full_bar[stage], 0, w0, h0 + p.rp_dir, n0);
           } else {
@@ -223,8 +218,8 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmDY, const __grid_constan
           if (p.xh) {
             // one box per (X block | X row): pixels w0-1 .. w0+Wb of the chunk's Hb rows, shifted by the filter row
             for (int b = 0; b < xh_live; ++b) {
-              const int cib = p.rowpair ? cib_base : cib_base + b;
-              const int xh_row = p.rowpair ? h0 + (p.rp_dir > 0 ? b + 1 : 0) - p.pad_h : h0 + rg - p.pad_h;
+              const int cib = rowpair ? cib_base : cib_base + b;
+              const int xh_row = rowpair ? h0 + (p.rp_dir > 0 ? b + 1 : 0) - p.pad_h : h0 + rg - p.pad_h;
               if (cib < p.cb0)
                 tma_load_4d(sb + b * kXhBox, &tmX0, &full_bar[stage], cib * 64, w0 - p.pad_w, xh_row, n0);
               else
@@ -233,10 +228,10 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmDY, const __grid_constan
           } else
           for (int j = 0; j < ncol_live; ++j) {
             // row-pair mode: group jg reads X row h0 + (jg + 1) - pad_h (filter row jg + 1 for the top half)
-            const int jg = p.rowpair ? j / grp_cols : 0;
+            const int jg = rowpair ? j / grp_cols : 0;
             const int cib = cib_base + (j - jg * grp_cols) / p.ksize;
             const int xw = p.xstride * w0 + (j % p.ksize) - p.pad_w;
-            const int xh = p.rowpair ? h0 + (p.rp_dir > 0 ? jg + 1 : 0) - p.pad_h : p.xstride * h0 + rg - p.pad_h;
+            const int xh = rowpair ? h0 + (p.rp_dir > 0 ? jg + 1 : 0) - p.pad_h : p.xstride * h0 + rg - p.pad_h;
             if (cib < p.cb0)
               tma_load_4d(sb + j * kBoxBytes, &tmX0, &full_bar[stage], cib * 64, xw, xh, n0);
             else
@@ -332,22 +327,6 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmDY, const __grid_constan
                 }
               }
             }
-          } else if (p.xh && p.tapn) {
-            const uint64_t desct = umma_desc_sw128(0, 128, 1024);      // N blocks = taps, one pixel (128 B) apart
-            const uint64_t desct_hi = desct & 0xFFFFFFFF00000000ull;
-            const uint32_t bt_lo = (uint32_t)desct + (b_addr >> 4);
-            const uint32_t idesct = umma_idesc_bf16(128, 192, 1, 1);
-#pragma unroll
-            for (int k = 0; k < kChunkPix / 16; ++k) {
-              if (k < nk) {
-                const uint64_t da = desc_hi | (uint64_t)(a_lo + 128u * k);
-                const uint32_t koff = (uint32_t)(((16 * k) / p.Wb) * (p.Wb + 2) + (16 * k) % p.Wb) * 8u;
-                for (int b = 0; b < xh_live; ++b)
-                  umma_bf16(tmem_base + (uint32_t)b * 192u, da,
-                            desct_hi | (uint64_t)(bt_lo + (uint32_t)b * (uint32_t)(kXhBox >> 4) + koff), idesct,
-                            (it | k) != 0 ? 1u : 0u);
-              }
-            }
           } else if (p.xh) {
             // three taps = three MMAs on the same halo boxes, B start shifted by one pixel (128 B = +8) per tap;
             // N = all boxes of the stage (kXhBox apart), accumulator columns [tap][box][64]
@@ -396,7 +375,7 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmDY, const __grid_constan
     // epilogue: row = output channel within the tile; columns = (column block, channel)
     const int quad = warp & 3;
     const int row = quad * 32 + lane;
-    const int co = (p.rowpair || p.fold == 2) ? (row & 63) : co_tile * 128 + row;
+    const int co = (rowpair || p.fold == 2) ? (row & 63) : co_tile * 128 + row;
     const bool valid = co < p.cout;
     float* out = p.ws + ((size_t)split * p.cout + (valid ? co : 0)) * ((size_t)p.taps * p.ctot);
     if (p.fold) out = p.ws + (size_t)split * 16 * p.cout * p.ctot;      // [phase][cout][2x2][ctot]
@@ -411,19 +390,18 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmDY, const __grid_constan
       int cib = cib_base + j / p.ksize;
       bool live = valid;
       if (p.fold) {
-        // accumulator columns are [q][box][64] ([box][q][64] with tapn); q = (b, tx) (fold 1) or the shift b + tx
-        // (fold 2: b = M half)
-        const int q = p.tapn ? j % 3 : j / xh_live;
+        // accumulator columns are [q][box][64]; q = (b, tx) (fold 1) or the shift b + tx (fold 2: b = M half)
+        const int q = j / xh_live;
         const int fb = p.fold == 1 ? q >> 1 : row >> 6;
         const int ftx = p.fold == 1 ? q & 1 : q - fb;
         live = valid && ftx >= 0 && ftx < 2;
-        cib = cib_base + (p.tapn ? j / 3 : j % xh_live);
+        cib = cib_base + j % xh_live;
         const int ph = (rg >> 1) * 2 + fb;
         tap = (ph * p.cout + (valid ? co : 0)) * 4 + (rg & 1) * 2 + (live ? ftx : 0);     // row index into [ph][co][tap]
       } else if (p.xh) {
         // accumulator columns are [tap s][box b][64]: b = X block (plain) or X row group (row-pair mode)
-        const int sx = p.tapn ? j % 3 : j / xh_live, b = p.tapn ? j / 3 : j % xh_live;
-        if (p.rowpair) {
+        const int sx = j / xh_live, b = j % xh_live;
+        if (rowpair) {
           const int fr = row < 64 ? b + 1 : (b == 0 ? 0 : -1);
           live = fr >= 0;
           tap = (fr < 0 ? 0 : fr) * 3 + sx;
@@ -432,7 +410,7 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap tmDY, const __grid_constan
           tap = rg * 3 + sx;
           cib = cib_base + b;
         }
-      } else if (p.rowpair) {
+      } else if (rowpair) {
         // group jg (X row h + jg + 1 - pad): dY row h -> filter row jg + 1, dY row h+1 -> filter row jg; the bottom
         // half of every group but the first repeats a filter row that the previous group already produced
         const int jg = j / grp_cols;
@@ -574,10 +552,8 @@ static int wgrad_plan(const b2_wgrad_args* a, WgradPlan* pl) {
   p.xstride = xstride;
   // 3x3: two 64-channel X blocks x 3 taps per CTA (N 384 as two MMAs that share the dY tile, 3 pipeline stages):
   // the kernel is bound by the L2 -> SM load rate, and this moves 64 KB per 6.3 MFLOP instead of 40 KB per 3.1
-  // (B200SEG_WG_CPB=1 selects the older one-block layout, N 192 with 5 stages)
-  const int cpb3 = env_switch("B200SEG_WG_CPB", 2) == 1 ? 1 : 2;
   p.debug_skip = env_switch("B200SEG_DEBUG_SKIP", 0);
-  p.cpb = a->ksize == 3 ? cpb3 : (a->ksize == 2 ? 2 : 4);
+  p.cpb = a->ksize == 1 ? 4 : 2;
   if (p.cpb > cbt) p.cpb = cbt;
   p.ncolb = p.ksize * p.cpb;
   pl->gy = p.ksize;
@@ -635,9 +611,8 @@ static int wgrad_plan(const b2_wgrad_args* a, WgradPlan* pl) {
   pl->count = (long long)a->cout * p.taps * p.ctot;
   {
     // X-halo mode: 3x3, unit stride, chunk = 64 consecutive pixels of one image row
-    const int want = env_switch("B200SEG_WG_XHALO", 1);
     // chunk = Hb rows of Wb pixels (64 x 1, 32 x 2, 16 x 4): the halo box has Hb rows of Wb + 2 pixels <= 72 rows
-    p.xh = (want != 0 && a->ksize == 3 && xstride == 1 && !a->custom_pad && p.Nb == 1 && p.Wb >= 16 &&
+    p.xh = (a->ksize == 3 && xstride == 1 && !a->custom_pad && p.Nb == 1 && p.Wb >= 16 &&
             (p.Wb + 2) * p.Hb * 128 <= kXhBox) ? 1 : 0;
     p.nbox = p.rowpair ? p.rowpair : p.cpb;
     if (p.fold) {
@@ -649,7 +624,6 @@ static int wgrad_plan(const b2_wgrad_args* a, WgradPlan* pl) {
   // CTA pairs: 3x3 halo mode, two Cout tiles per pair, each CTA holds one of the two X boxes
   p.pair = (env_switch("B200SEG_WG_PAIR", 1) != 0 && p.xh && (a->ksize == 3 || p.fold == 1) && !p.rowpair && p.fold != 2 &&
             p.cpb == 2 && a->cout % 256 == 0 && cbt % 2 == 0 && p.debug_skip == 0) ? 1 : 0;
-  p.tapn = (p.xh && !p.pair && p.fold != 1 && env_switch("B200SEG_WG_TAPN", 0) != 0) ? 1 : 0;
   p.b_stage_bytes = p.pair ? kXhBox : (p.xh ? p.nbox * kXhBox : p.ncolb * kBoxBytes);
   const int stage_bytes = p.a_bytes + p.b_stage_bytes;
   int stages = (200 * 1024) / stage_bytes;

@@ -202,11 +202,9 @@ def test_wgrad_folded_upconv_merged_rejects_narrow_images():
 
 
 @pytest.mark.parametrize("n,h,w,cin", [(2, 256, 256, 64), (2, 128, 128, 128), (1, 6, 128, 64)])
-def test_fprop_dgrad_rowpair_mode_matches_plain(n, h, w, cin):
-    """Cout = 64 row-pair mode of the implicit-GEMM kernel (B200SEG_FPROP_ROWPAIR=1: two output rows per tile, stacked
-    taps through a strided TMA box, N = 128 MMAs) against the default path and the fp32 reference, with bias, ReLU
-    and the BatchNorm-statistics epilogue."""
-    import os
+def test_fprop_dgrad_cout64_matches_fp32(n, h, w, cin):
+    """Cout = 64 3x3 fprop with bias, ReLU and the BatchNorm-statistics epilogue, and a dgrad into 64 channels, against
+    the fp32 reference; the statistics against fp64 sums of the stored output."""
     from b200seg import kernels as K
     g = torch.Generator(device="cuda").manual_seed(21)
     cout = 64
@@ -214,26 +212,15 @@ def test_fprop_dgrad_rowpair_mode_matches_plain(n, h, w, cin):
     wt = torch.randn(cout, cin, 3, 3, device="cuda", generator=g) / (cin * 9) ** 0.5
     b = torch.randn(cout, device="cuda", generator=g)
     wf, wd = K.pack_weights(wt)
-    dyv = nhwc(torch.randn(n, cout, h, w, device="cuda", generator=g))
     wt2 = torch.randn(cin, cout, 3, 3, device="cuda", generator=g) / (cout * 9) ** 0.5       # a conv whose dgrad has 64 ch
     _, wd2 = K.pack_weights(wt2)
     dy2 = nhwc(torch.randn(n, cin, h, w, device="cuda", generator=g))
-    res = {}
-    for mode in ("0", "1"):
-        os.environ["B200SEG_FPROP_ROWPAIR"] = mode
-        K.reload_switches()
-        try:
-            st = torch.zeros(2, cout, dtype=torch.float64, device="cuda")
-            y = K.conv_igemm(x, wf, cout, 3, bias=b, stats=st, relu=True)
-            dx = K.conv_igemm(dy2, wd2, cout, 3, dgrad=True)
-            res[mode] = (y, st, dx)
-        finally:
-            del os.environ["B200SEG_FPROP_ROWPAIR"]
-            K.reload_switches()
+    st = torch.zeros(2, cout, dtype=torch.float64, device="cuda")
+    y = K.conv_igemm(x, wf, cout, 3, bias=b, stats=st, relu=True)
+    dx = K.conv_igemm(dy2, wd2, cout, 3, dgrad=True)
     ref = torch.relu(F.conv2d(nchw(x), wt.to(torch.bfloat16).float(), b, padding=1))
-    assert rel(nchw(res["1"][0]), ref) < 4e-3
+    assert rel(nchw(y), ref) < 4e-3
     refd = F.conv_transpose2d(nchw(dy2), wt2.to(torch.bfloat16).float(), padding=1)
-    assert rel(nchw(res["1"][2]), refd) < 4e-3
-    assert rel(res["1"][0].float(), res["0"][0].float()) < 2e-3 and rel(res["1"][2].float(), res["0"][2].float()) < 2e-3
-    yf = res["1"][0].float().reshape(-1, cout)
-    assert rel(res["1"][1][0], yf.double().sum(0)) < 1e-5 and rel(res["1"][1][1], (yf.double() ** 2).sum(0)) < 1e-5
+    assert rel(nchw(dx), refd) < 4e-3
+    yf = y.float().reshape(-1, cout)
+    assert rel(st[0], yf.double().sum(0)) < 1e-5 and rel(st[1], (yf.double() ** 2).sum(0)) < 1e-5
