@@ -89,7 +89,7 @@ typedef struct b2_conv_args {
   void* y;                /* NHWC bf16 */
   int32_t ldy;
   const float* bias;      /* [cout] or NULL */
-  const void* addend;     /* optional NHWC bf16 [.., cout] added before rounding (NULL if unused) */
+  const void* addend;     /* optional NHWC bf16 [n, h, w, cout] added before rounding (NULL if unused; out_mul 1 only) */
   int32_t ldadd;
   double* stats;          /* optional [2][cout] (sum, sumsq), ACCUMULATED into (caller zeroes) */
   int32_t relu;

@@ -859,6 +859,9 @@ static int conv_igemm_launch(const b2_conv_args* a, cudaStream_t stream, const G
   B2_REQUIRE(a->ldy % 8 == 0 && (reinterpret_cast<uintptr_t>(a->y) & 15) == 0, B2_ERR_ALIGN, "y misaligned");
   B2_REQUIRE(a->addend == nullptr || (a->ldadd % 8 == 0 && (reinterpret_cast<uintptr_t>(a->addend) & 15) == 0),
              B2_ERR_ALIGN, "addend misaligned");
+  // the epilogue reads the addend at the conv-grid pixel, not at the placed output pixel: refuse what it cannot do
+  B2_REQUIRE(a->addend == nullptr || out_mul == 1, B2_ERR_SHAPE, "an addend with output placement (out_mul %d)",
+             out_mul);
   int tn;
   int rc = conv_tile_geometry(a->n, a->h, a->w, kTileM, &p.Wb, &p.Hb, &p.Nb, &p.tw, &p.th, &tn);
   if (rc) return rc;
