@@ -332,6 +332,49 @@ int b2_seg_counts(const float* z, const float* t, int32_t n, int64_t per_sample,
 int b2_logits_to_mask(const float* z, int64_t count, float thr_logit, uint8_t* mask, b2_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * Multi-class segmentation: z = fp32 NCHW logits [n][k][hw] (2 <= k <= 8, what b2_head_fwd writes), labels = class
+ * indices [n][hw], uint8 (label_bytes 1) or int64 (label_bytes 8).  A label equal to ignore_index takes part in
+ * nothing; a label outside [0, k) that is not ignore_index is INVALID: it is counted, takes part in nothing else, and
+ * makes the loss NaN (torch raises a device-side assert there; here the error surfaces without a host sync).
+ * argmax takes the lowest class index among equal maxima (torch.argmax).
+ *
+ * b2_ce_loss_fwd accumulates B2_CE_NSUMS(k) = 3 + 5k fp64 sums (caller zeroes; deterministic mode as b2_loss_fwd):
+ *   [B2_CE_LOSS]          sum w[y] * (logsumexp(z) - z_y)      w = `weight` (fp32 [k], NULL = all 1)
+ *   [B2_CE_WSUM]          sum w[y]
+ *   [B2_CE_PT(k) + c]     sum p_c [y = c]                      p = softmax(z)     (soft Dice intersection)
+ *   [B2_CE_P(k) + c]      sum p_c
+ *   [B2_CE_T(k) + c]      #[y = c]                             (sum over c = number of valid pixels)
+ *   [B2_CE_INTER(k) + c]  #[argmax = c and y = c]              (hard IoU of the training log)
+ *   [B2_CE_UNION(k) + c]  #[argmax = c or y = c]
+ *   [B2_CE_INVALID(k)]    #invalid labels
+ * ---------------------------------------------------------------------------------------------------------- */
+#define B2_CE_LOSS 0
+#define B2_CE_WSUM 1
+#define B2_CE_PT(k) (2)
+#define B2_CE_P(k) (2 + (k))
+#define B2_CE_T(k) (2 + 2 * (k))
+#define B2_CE_INTER(k) (2 + 3 * (k))
+#define B2_CE_UNION(k) (2 + 4 * (k))
+#define B2_CE_INVALID(k) (2 + 5 * (k))
+#define B2_CE_NSUMS(k) (3 + 5 * (k))
+int b2_ce_loss_fwd(const float* z, const void* labels, int32_t label_bytes, int32_t n, int32_t k, int64_t hw,
+                   const float* weight, int64_t ignore_index, double* sums, b2_stream_t stream);
+/* loss = w_ce * sums[LOSS] / sums[WSUM] + w_dice * (1 - mean over c = 1..k-1 of (2 PT_c + smooth) / (P_c + T_c + smooth));
+ * NaN when an invalid label was seen or no pixel is valid */
+int b2_ce_loss_finalize(const double* sums, int32_t k, float w_ce, float w_dice, float smooth, float* loss,
+                        b2_stream_t stream);
+/* dz = grad_out * d loss / d z (same layout as z; 0 on ignored and invalid pixels); grad_out: device scalar or NULL */
+int b2_ce_loss_bwd(const float* z, const void* labels, int32_t label_bytes, int32_t n, int32_t k, int64_t hw,
+                   const float* weight, int64_t ignore_index, const double* sums, float w_ce, float w_dice,
+                   float smooth, const float* grad_out, float* dz, b2_stream_t stream);
+/* counts[n][k][3] = {TP, #pred, #target} per sample and class, pred = argmax; ignored / invalid pixels excluded.
+ * The library zeroes counts. */
+int b2_seg_counts_mc(const float* z, const void* labels, int32_t label_bytes, int32_t n, int32_t k, int64_t hw,
+                     int64_t ignore_index, uint64_t* counts, b2_stream_t stream);
+/* labels[n][hw] = argmax over the k logits, uint8 */
+int b2_logits_to_labels(const float* z, int32_t n, int32_t k, int64_t hw, uint8_t* labels, b2_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------------------
  * Optimizer step (utils/helpers.py:333-335): clip_grad_norm_(max_norm) + AdamW over all parameters in two launches.
  * `refs` is a DEVICE array of tensor references (fp32, element-wise aligned layouts); block b processes elements
  * [block_chunk[b]*chunk_elems, ...) of tensor block_tensor[b].  `step` (device float) is incremented by
@@ -392,6 +435,13 @@ typedef struct b2_aug_params {
 int b2_seg_augment(const uint8_t* img, const uint8_t* mask, int32_t n, int32_t hs, int32_t ws, int32_t size,
                    const b2_aug_params* params, const float* mean3, const float* std3, int32_t mask_nearest_resize,
                    float* x, float* t, b2_stream_t stream);
+/* the same transform for multi-class label maps: the mask is resized and warped nearest-neighbour and flipped, and
+ * written as the uint8 label map labels[N][S][S] (no / 255); x is b2_seg_augment's.  The warp's border follows
+ * params.border for the labels as for the image (Albumentations' one border mode): constant 0 = background, or
+ * reflect-101 */
+int b2_seg_augment_labels(const uint8_t* img, const uint8_t* mask, int32_t n, int32_t hs, int32_t ws, int32_t size,
+                          const b2_aug_params* params, const float* mean3, const float* std3, float* x,
+                          uint8_t* labels, b2_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * Attention gate, eval mode, ONE kernel (north_star (2); AttentionUNet.py:29-54 / R2AttU_Net.py:61-86 with the three

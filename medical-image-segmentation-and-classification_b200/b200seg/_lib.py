@@ -151,6 +151,13 @@ SIGNATURES = {
     "b2_loss_bwd": (C.c_int, [_vp, _vp, _i64, _vp, _f32, _f32, _f32, _vp, _vp, _vp]),
     "b2_seg_counts": (C.c_int, [_vp, _vp, _i32, _i64, _f32, _f32, _vp, _vp]),
     "b2_logits_to_mask": (C.c_int, [_vp, _i64, _f32, _vp, _vp]),
+    "b2_ce_loss_fwd": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i64, _vp, _i64, _vp, _vp]),
+    "b2_ce_loss_finalize": (C.c_int, [_vp, _i32, _f32, _f32, _f32, _vp, _vp]),
+    "b2_ce_loss_bwd": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i64, _vp, _i64, _vp, _f32, _f32, _f32, _vp, _vp, _vp]),
+    "b2_seg_counts_mc": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i64, _i64, _vp, _vp]),
+    "b2_logits_to_labels": (C.c_int, [_vp, _i32, _i32, _i64, _vp, _vp]),
+    "b2_seg_augment_labels": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _vp, C.POINTER(_f32), C.POINTER(_f32), _vp,
+                                        _vp, _vp]),
 }
 
 _lib = None

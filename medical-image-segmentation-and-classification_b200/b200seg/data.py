@@ -74,7 +74,12 @@ class GpuSegAugment:
 
     def __init__(self, size=256, train=True, shift_limit=0.05, scale_limit=0.05, rotate_limit=15.0, p_ssr=0.7,
                  p_flip=0.5, brightness_limit=0.1, contrast_limit=0.1, p_bc=0.5, mean=IMAGENET_MEAN, std=IMAGENET_STD,
-                 border="constant", mask_nearest_resize=True, seed=None):
+                 border="constant", mask_nearest_resize=True, seed=None, labels=False):
+        """labels=True: the masks are multi-class label maps (class index per pixel); they are resized and warped
+        nearest-neighbour and returned as uint8 [N, S, S] class indices instead of fp32 [N, 1, S, S] in {0, 1}"""
+        if labels and not mask_nearest_resize:
+            raise ValueError("label maps are resized nearest-neighbour: labels=True needs mask_nearest_resize=True")
+        self.labels = bool(labels)
         self.size, self.train = int(size), bool(train)
         self.shift_limit, self.scale_limit, self.rotate_limit, self.p_ssr = shift_limit, scale_limit, rotate_limit, p_ssr
         self.p_flip, self.brightness_limit, self.contrast_limit, self.p_bc = p_flip, brightness_limit, contrast_limit, p_bc
@@ -102,7 +107,7 @@ class GpuSegAugment:
 
     def __call__(self, img_u8, mask_u8, samples=None, device=None):
         """img_u8 uint8 [N, Hs, Ws, 3], mask_u8 uint8 [N, Hs, Ws] (or [N, Hs, Ws, 1]); host or device tensors.
-        Returns (x fp32 [N, 3, S, S], t fp32 [N, 1, S, S]) on the device."""
+        Returns (x fp32 [N, 3, S, S], t fp32 [N, 1, S, S]) on the device; with labels=True t is uint8 [N, S, S]."""
         assert img_u8.dtype == torch.uint8 and mask_u8.dtype == torch.uint8 and img_u8.dim() == 4 and img_u8.shape[3] == 3
         if mask_u8.dim() == 4:
             mask_u8 = mask_u8[..., 0]
@@ -115,6 +120,11 @@ class GpuSegAugment:
         prm = torch.from_numpy(pack_params(self.size, samples, self.border)).to(dev, non_blocking=True)
         S = self.size
         x = torch.empty((n, 3, S, S), dtype=torch.float32, device=dev)
+        if self.labels:
+            y = torch.empty((n, S, S), dtype=torch.uint8, device=dev)
+            call("b2_seg_augment_labels", _p(img_d), _p(msk_d), n, hs, ws, S, _p(prm), self.mean, self.std, _p(x), _p(y),
+                 _stream())
+            return x, y
         t = torch.empty((n, 1, S, S), dtype=torch.float32, device=dev)
         call("b2_seg_augment", _p(img_d), _p(msk_d), n, hs, ws, S, _p(prm), self.mean, self.std,
              int(self.mask_nearest_resize), _p(x), _p(t), _stream())

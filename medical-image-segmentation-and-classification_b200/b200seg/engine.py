@@ -31,19 +31,29 @@ class GraphedTrainStep:
 
     `loss_weights` = (w_bce, w_dice, smooth) of b200seg::seg_loss (BCEWithLogits = (1, 0, 1), helpers.py:245;
     CombinedLoss = (0.5, 0.5, 1), clip_seg_finetuner.py:61-74).
+    `loss="ce"`: multi-class training on K >= 2 logit channels and integer label maps (uint8 / int64 [N, H, W]) through
+    b200seg::seg_loss_ce; `loss_weights` then means (w_ce, w_dice, smooth), `class_weight` (K floats) and
+    `ignore_index` have nn.CrossEntropyLoss's meaning.
     """
 
     def __init__(self, model: torch.nn.Module, optimizer, reducer=None, loss_weights=(1.0, 0.0, 1.0), graph: bool = True,
                  warmup: int = 3, max_graphs: int = 2, wgrad_overlap: Optional[bool] = None,
-                 clip_fn: Optional[Callable[[], None]] = None):
+                 clip_fn: Optional[Callable[[], None]] = None, loss: str = "bce", class_weight=None,
+                 ignore_index: int = -100):
+        if loss not in ("bce", "ce"):
+            raise ValueError(f"loss must be 'bce' or 'ce', got {loss!r}")
         self.model, self.optimizer, self.reducer = model, optimizer, reducer
         self.loss_weights = tuple(float(v) for v in loss_weights)
+        self.loss = loss
+        self.ignore_index = int(ignore_index)
         self.use_graph = bool(graph)
         self.warmup = max(int(warmup), 1)
         self.max_graphs = int(max_graphs)
         self.wgrad_overlap = wgrad_overlap
         self.clip_fn = clip_fn                      # for non-fused optimizers: called between backward and step
         self.device = next(model.parameters()).device
+        self.class_weight = None if class_weight is None else \
+            torch.as_tensor(class_weight, dtype=torch.float32).to(self.device).contiguous()
         self.stream = torch.cuda.Stream(device=self.device)
         self._seen: Dict[Tuple, int] = {}
         self._graphs: Dict[Tuple, Tuple] = {}       # shape key -> (graph, x_static, t_static, loss_static, launches)
@@ -60,7 +70,10 @@ class GraphedTrainStep:
             logits = self.model(x)
         if logits.dim() == 3:
             logits = logits.unsqueeze(1)            # helpers.py:323-324
-        loss, _sums = ops.seg_loss(logits, t, *self.loss_weights)
+        if self.loss == "ce":
+            loss, _sums = ops.seg_loss_ce(logits, t, self.class_weight, self.ignore_index, *self.loss_weights)
+        else:
+            loss, _sums = ops.seg_loss(logits, t, *self.loss_weights)
         loss.backward()
         if self.reducer is not None:
             self.reducer.finish()

@@ -1000,3 +1000,88 @@ def loss_bwd(z, t, sums, grad_out, w_bce=1.0, w_dice=0.0, smooth=1.0):
     call("b2_loss_bwd", _p(z), _p(t), z.numel(), _p(sums), float(w_bce), float(w_dice), float(smooth),
          _p(grad_out), _p(dz), _stream())
     return dz
+
+
+# ----------------------------------------------------------------------------------------------------------
+# multi-class: softmax cross-entropy + soft Dice, per-class counts, argmax label map (csrc/loss_mc.cu)
+# ----------------------------------------------------------------------------------------------------------
+MAX_CLASSES = 8
+
+
+def ce_nsums(k):
+    """number of fp64 sums b2_ce_loss_fwd accumulates for k classes (B2_CE_NSUMS)"""
+    return 3 + 5 * k
+
+
+def ce_sums_fields(sums, k):
+    """named views of the b2_ce_loss_fwd sums (layout: include/b200seg.h, B2_CE_*)"""
+    return {"loss": sums[0], "wsum": sums[1], "pt": sums[2:2 + k], "p": sums[2 + k:2 + 2 * k],
+            "t": sums[2 + 2 * k:2 + 3 * k], "inter": sums[2 + 3 * k:2 + 4 * k], "union": sums[2 + 4 * k:2 + 5 * k],
+            "invalid": sums[2 + 5 * k]}
+
+
+def _mc_args(z, labels):
+    """(n, k, hw, label_bytes) of fp32 NCHW logits [N, K, H, W] and uint8 / int64 labels [N, H, W] or [N, 1, H, W]"""
+    assert z.dtype == torch.float32 and z.is_contiguous() and z.dim() == 4 and z.is_cuda, (z.dtype, z.shape)
+    n, k, h, w = z.shape
+    if not 2 <= k <= MAX_CLASSES:
+        raise ValueError(f"multi-class kernels take 2..{MAX_CLASSES} classes, the logits have {k} channels")
+    if labels.dtype not in (torch.uint8, torch.int64):
+        raise TypeError(f"labels must be uint8 or int64 class indices, got {labels.dtype}")
+    if labels.numel() != n * h * w or labels.shape[0] != n or labels.shape[-2:] != (h, w):
+        raise ValueError(f"labels {tuple(labels.shape)} do not match logits {tuple(z.shape)}")
+    assert labels.is_contiguous() and labels.device == z.device
+    return n, k, h * w, labels.element_size()
+
+
+def _mc_weight(weight, z, k):
+    """the class-weight vector the kernels read with device loads: fp32, contiguous, K entries, on the logits' device"""
+    if weight is None:
+        return
+    if weight.device != z.device:
+        raise ValueError(f"class weight is on {weight.device}, the logits on {z.device}")
+    if weight.dtype != torch.float32 or not weight.is_contiguous() or weight.numel() != k:
+        raise ValueError(f"class weight must be a contiguous fp32 vector of {k} entries, got {weight.dtype} "
+                         f"{tuple(weight.shape)}")
+
+
+def ce_loss_fwd(z, labels, weight=None, ignore_index=-100, w_ce=1.0, w_dice=0.0, smooth=1.0):
+    """-> (loss fp32 scalar, sums fp64 [3 + 5K]); loss is NaN when a label is outside [0, K) and not ignore_index, or
+    when no pixel is valid"""
+    n, k, hw, lb = _mc_args(z, labels)
+    _mc_weight(weight, z, k)
+    sums = zeros_out((ce_nsums(k),), torch.float64, z.device)   # an output of seg_loss_ce: not arena memory
+    loss = torch.empty((), dtype=torch.float32, device=z.device)
+    call("b2_ce_loss_fwd", _p(z), _p(labels), lb, n, k, hw, _p(weight), int(ignore_index), _p(sums), _stream())
+    call("b2_ce_loss_finalize", _p(sums), k, float(w_ce), float(w_dice), float(smooth), _p(loss), _stream())
+    return loss, sums
+
+
+def ce_loss_bwd(z, labels, weight, ignore_index, sums, grad_out, w_ce=1.0, w_dice=0.0, smooth=1.0):
+    n, k, hw, lb = _mc_args(z, labels)
+    _mc_weight(weight, z, k)
+    assert sums.dtype == torch.float64 and sums.numel() == ce_nsums(k) and sums.device == z.device
+    assert grad_out is None or (grad_out.dtype == torch.float32 and grad_out.device == z.device)
+    dz = torch.empty_like(z)
+    call("b2_ce_loss_bwd", _p(z), _p(labels), lb, n, k, hw, _p(weight), int(ignore_index), _p(sums), float(w_ce),
+         float(w_dice), float(smooth), _p(grad_out), _p(dz), _stream())
+    return dz
+
+
+def seg_counts_mc(z, labels, ignore_index=-100):
+    """fp32 logits [N, K, H, W] + labels -> int64 [N, K, 3] = (TP, #pred, #target) per sample and class, pred = argmax"""
+    n, k, hw, lb = _mc_args(z, labels)
+    counts = torch.empty((n, k, 3), dtype=torch.int64, device=z.device)
+    call("b2_seg_counts_mc", _p(z), _p(labels), lb, n, k, hw, int(ignore_index), _p(counts), _stream())
+    return counts
+
+
+def logits_to_labels(z):
+    """fp32 logits [N, K, H, W] -> uint8 label map [N, H, W] (argmax, first maximum on ties)"""
+    assert z.dtype == torch.float32 and z.is_contiguous() and z.dim() == 4 and z.is_cuda
+    n, k, h, w = z.shape
+    if not 2 <= k <= MAX_CLASSES:
+        raise ValueError(f"multi-class kernels take 2..{MAX_CLASSES} classes, the logits have {k} channels")
+    out = torch.empty((n, h, w), dtype=torch.uint8, device=z.device)
+    call("b2_logits_to_labels", _p(z), n, k, h * w, _p(out), _stream())
+    return out

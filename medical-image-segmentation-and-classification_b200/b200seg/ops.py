@@ -753,3 +753,47 @@ def _loss_backward(ctx, g, _gs):
 
 
 seg_loss.register_autograd(_loss_backward, setup_context=_loss_setup)
+
+
+# ----------------------------------------------------------------------------------------------------------
+# multi-class loss: w_ce * CrossEntropy(weight, ignore_index) + w_dice * (1 - mean foreground soft Dice)
+# (nn.CrossEntropyLoss semantics; w_ce = w_dice = 0.5 mirrors CombinedLoss, clip_seg_finetuner.py:61-74)
+# ----------------------------------------------------------------------------------------------------------
+@custom_op("b200seg::seg_loss_ce", mutates_args=())
+def seg_loss_ce(logits: Tensor, labels: Tensor, weight: Optional[Tensor], ignore_index: int, w_ce: float,
+                w_dice: float, smooth: float) -> Tuple[Tensor, Tensor]:
+    """logits fp32 [N, K, H, W], labels uint8 / int64 [N, H, W] (or [N, 1, H, W]) -> (scalar loss fp32, sums fp64
+    [3 + 5K], layout kernels.ce_sums_fields).  The loss is NaN when a label is neither in [0, K) nor ignore_index."""
+    return K.ce_loss_fwd(_c(logits.float()), _c(labels), _c(weight), ignore_index, w_ce, w_dice, smooth)
+
+
+@seg_loss_ce.register_fake
+def _(logits, labels, weight, ignore_index, w_ce, w_dice, smooth):
+    return logits.new_empty((), dtype=torch.float32), logits.new_empty((K.ce_nsums(logits.shape[1]),), dtype=_F64)
+
+
+@custom_op("b200seg::seg_loss_ce_bwd", mutates_args=())
+def seg_loss_ce_bwd(grad_out: Tensor, logits: Tensor, labels: Tensor, weight: Optional[Tensor], ignore_index: int,
+                    sums: Tensor, w_ce: float, w_dice: float, smooth: float) -> Tensor:
+    return K.ce_loss_bwd(_c(logits.float()), _c(labels), _c(weight), ignore_index, sums, _c(grad_out.float()), w_ce,
+                         w_dice, smooth)
+
+
+@seg_loss_ce_bwd.register_fake
+def _(grad_out, logits, labels, weight, ignore_index, sums, w_ce, w_dice, smooth):
+    return torch.empty_like(logits, dtype=torch.float32)
+
+
+def _loss_ce_setup(ctx, inputs, output):
+    ctx.set_materialize_grads(False)
+    logits, labels, weight, ctx.ignore_index, ctx.w_ce, ctx.w_dice, ctx.smooth = inputs
+    ctx.save_for_backward(logits, labels, weight, output[1])
+
+
+def _loss_ce_backward(ctx, g, _gs):
+    logits, labels, weight, sums = ctx.saved_tensors
+    dz = seg_loss_ce_bwd(g, logits, labels, weight, ctx.ignore_index, sums, ctx.w_ce, ctx.w_dice, ctx.smooth)
+    return dz.view_as(logits), None, None, None, None, None, None
+
+
+seg_loss_ce.register_autograd(_loss_ce_backward, setup_context=_loss_ce_setup)

@@ -11,7 +11,9 @@ Differences from the reference, all forced by the B200 path and listed in DESIGN
     and replayed (engine.GraphedTrainStep; B200SEG_TRAIN_GRAPH=0 launches eagerly), and CPU batches are staged through
     pinned memory and copied on a copy stream while the previous step computes (engine.PinnedPrefetcher);
   * B200SEG_TRAIN_LOG=<file> appends one JSON line per epoch (losses, IoU, images/s of the training loop, graph
-    replays) next to the reference's per-epoch print (SURVEY.md §5, metrics / logging).
+    replays) next to the reference's per-epoch print (SURVEY.md §5, metrics / logging);
+  * train(loss="ce" | "ce+dice") trains K >= 2 mutually exclusive classes on integer label maps with the fused
+    b200seg::seg_loss_ce op (softmax cross-entropy, + soft Dice over the foreground classes for "ce+dice").
 """
 from __future__ import annotations
 
@@ -57,11 +59,22 @@ def _dataset_len(dl, fallback):
         return fallback
 
 
+# multi-class loss modes -> (w_ce, w_dice, smooth) of b200seg::seg_loss_ce; "ce+dice" weighs like CombinedLoss
+_CE_MODES = {"ce": (1.0, 0.0, 1.0), "ce+dice": (0.5, 0.5, 1.0)}
+
+
 def train(model, train_dl, val_dl, device, epochs, lr, name, save_dir, seg=False, cls_head_name=None,
-          reducer=None, log=print):
-    """helpers.py:231-412, segmentation branch.  Returns the best validation loss."""
+          reducer=None, log=print, loss="bce", class_weight=None, ignore_index=-100):
+    """helpers.py:231-412, segmentation branch.  Returns the best validation loss.
+
+    loss="bce" (default) is the reference's BCEWithLogits on one mask channel.  "ce" / "ce+dice" train the model's K >= 2
+    output channels as mutually exclusive classes on integer label maps (uint8 / int64 [N, H, W]; `class_weight` and
+    `ignore_index` as in nn.CrossEntropyLoss); the printed IoU is then the mean over the foreground classes 1..K-1 of
+    inter / union per validation batch."""
     if not seg:
         raise NotImplementedError("b200seg.train covers the segmentation path only (seg=True)")
+    if loss != "bce" and loss not in _CE_MODES:
+        raise ValueError(f"loss must be 'bce', 'ce' or 'ce+dice', got {loss!r}")
     device = torch.device(device)
     model = model.to(device, memory_format=torch.channels_last)            # helpers.py:243
     from .. import kernels as K
@@ -77,8 +90,13 @@ def train(model, train_dl, val_dl, device, epochs, lr, name, save_dir, seg=False
     patience, patience_counter = 10, 0
     from ..engine import GraphedTrainStep, PinnedPrefetcher
     on_gpu = device.type == "cuda"
-    stepper = GraphedTrainStep(model, optimizer, reducer=reducer, loss_weights=(1.0, 0.0, 1.0),     # helpers.py:245
-                               graph=on_gpu and os.environ.get("B200SEG_TRAIN_GRAPH", "1") != "0")
+    graph = on_gpu and os.environ.get("B200SEG_TRAIN_GRAPH", "1") != "0"
+    if loss == "bce":
+        stepper = GraphedTrainStep(model, optimizer, reducer=reducer, loss_weights=(1.0, 0.0, 1.0),  # helpers.py:245
+                                   graph=graph)
+    else:
+        stepper = GraphedTrainStep(model, optimizer, reducer=reducer, loss_weights=_CE_MODES[loss], graph=graph,
+                                   loss="ce", class_weight=class_weight, ignore_index=ignore_index)
     train.last_stepper = stepper          # introspection for tests / tools: replays, eager steps, capture errors
     start_time = time.time()
 
@@ -94,8 +112,8 @@ def train(model, train_dl, val_dl, device, epochs, lr, name, save_dir, seg=False
                     x, y = x.to(device, non_blocking=True), y.to(device, non_blocking=True)
                 # zero_grad -> forward -> BCEWithLogits -> backward -> (all-reduce) -> clip_grad_norm_(1.0) + AdamW,
                 # replayed from a CUDA graph after the first few (eager) steps of each batch shape
-                loss = stepper(x.float(), y.float())
-                running += loss.detach().double() * x.size(0)
+                step_loss = stepper(x.float(), y.float()) if loss == "bce" else stepper(x.float(), y)
+                running += step_loss.detach().double() * x.size(0)
                 seen += x.size(0)
             running_sum = float(running)              # the epoch's one host sync of the training loop
             train_s = time.time() - t_epoch
@@ -110,9 +128,15 @@ def train(model, train_dl, val_dl, device, epochs, lr, name, save_dir, seg=False
                     out = model(x)
                     if out.dim() == 3:
                         out = out.unsqueeze(1)
-                    loss, sums = ops.seg_loss(out, y, 1.0, 0.0, 1.0)
-                    val_loss += loss.double() * x.size(0)
-                    val_iou += sums[4] / (sums[5] + 1e-7)                     # helpers.py:223-227 per batch
+                    if loss == "bce":
+                        vloss, sums = ops.seg_loss(out, y, 1.0, 0.0, 1.0)
+                        val_loss += vloss.double() * x.size(0)
+                        val_iou += sums[4] / (sums[5] + 1e-7)                 # helpers.py:223-227 per batch
+                    else:
+                        vloss, sums = ops.seg_loss_ce(out, y, stepper.class_weight, ignore_index, *_CE_MODES[loss])
+                        val_loss += vloss.double() * x.size(0)
+                        f = K.ce_sums_fields(sums, out.shape[1])
+                        val_iou += (f["inter"][1:] / (f["union"][1:] + 1e-7)).mean()   # foreground classes
                     n_val += x.size(0)
                     n_batches += 1
             if reducer is not None:

@@ -36,6 +36,28 @@ def xray_batch(n, h=256, w=256, seed=0, device="cpu", dtype=torch.float32):
     return x.contiguous().to(device=device, dtype=dtype), mask.contiguous().to(device=device, dtype=dtype)
 
 
+def xray_batch_multiclass(n, h=256, w=256, seed=0, device="cpu", dtype=torch.float32):
+    """xray_batch's image with a 3-class label map uint8 [N, H, W]: 0 background, 1 lung, 2 a lesion — a seeded
+    ellipse around a point of one lung's mask, clipped to that mask (the background / lung / infection maps of the
+    reference's dataset family)."""
+    x, mask = xray_batch(n, h, w, seed=seed, device="cpu", dtype=torch.float32)
+    lung = mask[:, 0] > 0.5
+    labels = lung.to(torch.uint8)
+    g = torch.Generator().manual_seed(seed + 7919)
+    ys = torch.linspace(-1, 1, h).view(h, 1)
+    xs = torch.linspace(-1, 1, w).view(1, w)
+    for i in range(n):
+        idx = lung[i].flatten().nonzero()[:, 0]
+        if idx.numel() == 0:
+            continue
+        c = int(idx[int(torch.randint(idx.numel(), (1,), generator=g))])
+        cy, cx = float(ys[c // w, 0]), float(xs[0, c % w])
+        ry, rx = (0.1 + 0.1 * torch.rand(2, generator=g)).tolist()
+        lesion = ((ys - cy) / ry) ** 2 + ((xs - cx) / rx) ** 2 <= 1.0
+        labels[i][lesion & lung[i]] = 2
+    return x.to(device=device, dtype=dtype), labels.contiguous().to(device)
+
+
 def noise_batch(n, h=256, w=256, seed=1234, device="cpu", dtype=torch.float32):
     g = torch.Generator().manual_seed(seed)
     x = torch.randn(n, 3, h, w, generator=g)

@@ -43,6 +43,27 @@ def metrics_from_counts(counts, per_sample):
     return {k: v * 100 for k, v in zip(METRIC_KEYS, vals)}
 
 
+# per-class keys of the multi-class report: f"{key}_c{k}" for every class k
+CLASS_METRIC_KEYS = ("iou", "dice", "precision", "recall", "f1")
+
+
+def metrics_from_counts_mc(counts):
+    """int64 [N, K, 3] = (TP, #pred, #target) per sample and class (kernels.seg_counts_mc) -> dict of fp64 tensors in
+    percent: per-class [N, K] entries for CLASS_METRIC_KEYS and the per-sample pixel accuracy [N] = sum TP / #valid
+    pixels; the reference's 1e-7 guards, so a class absent from both prediction and label scores 100"""
+    c = counts.double()
+    tp, npred, ntgt = c[..., 0], c[..., 1], c[..., 2]
+    eps = 1e-7
+    iou = (tp + eps) / (npred + ntgt - tp + eps)
+    dice = (2.0 * tp + eps) / (npred + ntgt + eps)
+    precision = (tp + eps) / (npred + eps)
+    recall = (tp + eps) / (ntgt + eps)
+    f1 = 2 * (precision * recall) / (precision + recall + eps)
+    out = {k: v * 100 for k, v in zip(CLASS_METRIC_KEYS, (iou, dice, precision, recall, f1))}
+    out["pixel_accuracy"] = tp.sum(1) / ntgt.sum(1).clamp_min(1) * 100
+    return out
+
+
 def _single(pred, target, threshold):
     p = pred.detach().float().reshape(1, -1).contiguous()
     t = target.detach().float().reshape(1, -1).contiguous()
@@ -70,11 +91,17 @@ def calculate_segmentation_metrics(pred, target, threshold=0.5):
     return _single(pred, target, threshold)
 
 
-def test_segmentation_model(model, test_loader, device, model_name, log=print):
-    """tester.py:249-312: average of the per-sample metrics over the test set."""
+def test_segmentation_model(model, test_loader, device, model_name, log=print, ignore_index=-100):
+    """tester.py:249-312: average of the per-sample metrics over the test set.
+
+    Multi-class: when the masks are integer label maps and the model returns K >= 2 channels, pred = argmax and the
+    metrics are counted per sample and class (kernels.seg_counts_mc; `ignore_index` pixels excluded).  The six keys are
+    then the means over the foreground classes 1..K-1 (pixel accuracy: sum TP / valid pixels), and f"{key}_c{k}" holds
+    each class's own average."""
     model.eval()
     device = torch.device(device)
-    totals = torch.zeros(len(METRIC_KEYS), dtype=torch.float64, device=device)
+    totals = None
+    multiclass = None                                        # which counting the first batch selected
     num_samples = 0
     log(f"\n{'=' * 60}")
     log(f"Testing Segmentation Model: {model_name}")
@@ -86,12 +113,36 @@ def test_segmentation_model(model, test_loader, device, model_name, log=print):
             outputs = model(images)
             if outputs.dim() == 3:
                 outputs = outputs.unsqueeze(1)
-            counts = segmentation_counts(outputs, masks.reshape(outputs.shape), 0.5)
-            m = metrics_from_counts(counts, outputs[0].numel())
-            totals += torch.stack([m[k].sum() for k in METRIC_KEYS])
+            batch_mc = outputs.shape[1] >= 2 and not masks.is_floating_point()
+            if multiclass is None:
+                multiclass = batch_mc
+            elif batch_mc != multiclass:
+                raise ValueError("test loader mixes integer label maps and float masks")
+            if batch_mc:
+                z = outputs.detach().float().contiguous()
+                m = metrics_from_counts_mc(K.seg_counts_mc(z, masks.contiguous(), ignore_index))
+                batch = torch.cat([m["pixel_accuracy"].sum().view(1)] + [m[k].sum(0) for k in CLASS_METRIC_KEYS])
+            else:
+                counts = segmentation_counts(outputs, masks.reshape(outputs.shape), 0.5)
+                m = metrics_from_counts(counts, outputs[0].numel())
+                batch = torch.stack([m[k].sum() for k in METRIC_KEYS])
+            if totals is None:
+                totals = torch.zeros_like(batch)
+            totals += batch
             num_samples += outputs.size(0)
+    if totals is None:
+        totals = torch.zeros(len(METRIC_KEYS), dtype=torch.float64, device=device)
     avg = (totals / max(num_samples, 1)).tolist()            # the only host sync
-    avg_metrics = dict(zip(METRIC_KEYS, avg))
+    if not multiclass:
+        avg_metrics = dict(zip(METRIC_KEYS, avg))
+    else:                                                    # [pixel accuracy, then K values per class metric]
+        ncls = (len(avg) - 1) // len(CLASS_METRIC_KEYS)
+        per_class = {key: avg[1 + i * ncls:1 + (i + 1) * ncls] for i, key in enumerate(CLASS_METRIC_KEYS)}
+        avg_metrics = {key: sum(v[1:]) / (ncls - 1) for key, v in per_class.items()}
+        avg_metrics["pixel_accuracy"] = avg[0]
+        avg_metrics = {key: avg_metrics[key] for key in METRIC_KEYS}
+        for key, v in per_class.items():
+            avg_metrics.update({f"{key}_c{k}": v[k] for k in range(ncls)})
     log(f"\n{model_name} Test Results:")
     log(f"{'-' * 60}")
     log(f"IoU (Jaccard):     {avg_metrics['iou']:.2f}%")
@@ -125,3 +176,20 @@ def predict_mask(model, img_tensor, threshold=0.5, precision=None):
     if mask.shape[0] == 1:
         mask = mask[0]
     return mask.numpy()
+
+
+def predict_labels(model, img_tensor, precision=None):
+    """Multi-class counterpart of predict_mask: logits [N, K, H, W] (K >= 2) -> uint8 label map = argmax over the
+    classes (first maximum on ties, as torch.argmax) on the host; [H, W] for one image, [N, H, W] otherwise.
+    precision="fp32": the fp32 parity mode (ops_fp32.py); None: b200seg.get_precision()."""
+    import contextlib
+    from .. import ops_fp32
+    model.eval()
+    dev = next(model.parameters()).device
+    with torch.no_grad(), (ops_fp32.precision(precision) if precision else contextlib.nullcontext()):
+        logits = model(img_tensor.to(dev)).float().contiguous()
+        labels = K.logits_to_labels(logits)
+    labels = labels.cpu()
+    if labels.shape[0] == 1:
+        labels = labels[0]
+    return labels.numpy()

@@ -55,10 +55,12 @@ __device__ __forceinline__ float resized_mask(const uint8_t* __restrict__ msk, i
   return resized_u8(msk, hs, ws, 1, 0, yy, xx, sy, sx);
 }
 
+// kLabels: the mask is a class-index map (nearest resize, written as uint8 to `t`); otherwise {0, 255} -> fp32 {0, 1}
+template <bool kLabels>
 __global__ void __launch_bounds__(256) seg_augment_kernel(const uint8_t* __restrict__ img, const uint8_t* __restrict__ msk,
                                                           int n, int hs, int ws, int S, const AugSample* __restrict__ prm,
                                                           float3 mean, float3 inv_std, int mask_nearest_resize,
-                                                          float* __restrict__ x, float* __restrict__ t) {
+                                                          float* __restrict__ x, void* __restrict__ t) {
   const long long total = (long long)n * S * S;
   const float sy = (float)hs / S, sx = (float)ws / S;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
@@ -106,17 +108,14 @@ __global__ void __launch_bounds__(256) seg_augment_kernel(const uint8_t* __restr
     x[((long long)b * 3 + 0) * plane + o] = (rgb[0] * (1.f / 255.f) - mean.x) * inv_std.x;
     x[((long long)b * 3 + 1) * plane + o] = (rgb[1] * (1.f / 255.f) - mean.y) * inv_std.y;
     x[((long long)b * 3 + 2) * plane + o] = (rgb[2] * (1.f / 255.f) - mean.z) * inv_std.z;
-    t[(long long)b * plane + o] = mv * (1.f / 255.f);
+    if constexpr (kLabels) static_cast<uint8_t*>(t)[(long long)b * plane + o] = (uint8_t)mv;
+    else static_cast<float*>(t)[(long long)b * plane + o] = mv * (1.f / 255.f);
   }
 }
 
-}  // namespace b2
-
-using namespace b2;
-
-extern "C" int b2_seg_augment(const uint8_t* img, const uint8_t* mask, int32_t n, int32_t hs, int32_t ws, int32_t size,
-                              const b2_aug_params* params, const float* mean3, const float* std3,
-                              int32_t mask_nearest_resize, float* x, float* t, b2_stream_t stream) {
+static int seg_augment(bool labels, const uint8_t* img, const uint8_t* mask, int32_t n, int32_t hs, int32_t ws,
+                       int32_t size, const b2_aug_params* params, const float* mean3, const float* std3,
+                       int32_t mask_nearest_resize, float* x, void* t, b2_stream_t stream) {
   static_assert(sizeof(AugSample) == sizeof(b2_aug_params), "AugSample must mirror b2_aug_params");
   int rc = b2_arch_check();
   if (rc) return rc;
@@ -126,9 +125,31 @@ extern "C" int b2_seg_augment(const uint8_t* img, const uint8_t* mask, int32_t n
   long long grid = (total + 255) / 256;
   const long long cap = (long long)num_sms() * 16;
   if (grid > cap) grid = cap;
-  seg_augment_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(
-      img, mask, n, hs, ws, size, reinterpret_cast<const AugSample*>(params), make_float3(mean3[0], mean3[1], mean3[2]),
-      make_float3(1.f / std3[0], 1.f / std3[1], 1.f / std3[2]), mask_nearest_resize, x, t);
+  const float3 mean = make_float3(mean3[0], mean3[1], mean3[2]);
+  const float3 inv_std = make_float3(1.f / std3[0], 1.f / std3[1], 1.f / std3[2]);
+  const AugSample* prm = reinterpret_cast<const AugSample*>(params);
+  if (labels)
+    seg_augment_kernel<true><<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(img, mask, n, hs, ws, size, prm, mean,
+                                                                              inv_std, mask_nearest_resize, x, t);
+  else
+    seg_augment_kernel<false><<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(img, mask, n, hs, ws, size, prm, mean,
+                                                                               inv_std, mask_nearest_resize, x, t);
   B2_LAUNCH_CHECK();
   return B2_OK;
+}
+
+}  // namespace b2
+
+using namespace b2;
+
+extern "C" int b2_seg_augment(const uint8_t* img, const uint8_t* mask, int32_t n, int32_t hs, int32_t ws, int32_t size,
+                              const b2_aug_params* params, const float* mean3, const float* std3,
+                              int32_t mask_nearest_resize, float* x, float* t, b2_stream_t stream) {
+  return seg_augment(false, img, mask, n, hs, ws, size, params, mean3, std3, mask_nearest_resize, x, t, stream);
+}
+
+extern "C" int b2_seg_augment_labels(const uint8_t* img, const uint8_t* mask, int32_t n, int32_t hs, int32_t ws,
+                                     int32_t size, const b2_aug_params* params, const float* mean3, const float* std3,
+                                     float* x, uint8_t* labels, b2_stream_t stream) {
+  return seg_augment(true, img, mask, n, hs, ws, size, params, mean3, std3, 1, x, labels, stream);
 }
